@@ -7,6 +7,7 @@ data-path collective.  A step is one pass of the hot path over that resident bat
 reference-precision (fp64) path on the same records instead.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                          # also save the last timed step's outputs (.npy)
     python bench.py --impl reference ...                            # CPU port of the reference (oracle), host cores
     torchrun --nproc-per-node N bench.py --gpus N ...               # one rank per GPU
 
@@ -22,6 +23,8 @@ Rank 0 prints ONE JSON line (contract in the task statement):
   configs      device-timed secondary configurations run after the headline: BASELINE configs[3] share (order 6,
                8 ch x 2^22) and, for N > 1, configs[4]-shaped band sharding of ONE long record (order 12) with its single
                NCCL all-reduce of the total power
+  dump_outputs (with --dump-outputs DIR) the files written to DIR: what the last timed step returned to its caller on
+               rank 0, so that two builds run with the same arguments can be compared output for output
 """
 import argparse
 import hashlib
@@ -314,6 +317,44 @@ def checks_rank0(torch, cwt_entropy, x, power, info, r, n, n_bands):
     return out
 
 
+DUMP_PLANE_BYTES = 24 << 20       # per [C, B, N] plane: power + info + the per-band arrays stay under 64 MB in all
+
+
+def plane_sample_index(shape, itemsize, seed=0):
+    """Flat indices of the cells of a [C, B, N] plane that --dump-outputs saves: None (the whole plane) when it fits
+    DUMP_PLANE_BYTES, else a uniform sample drawn from a fixed seed (sorted, repeats dropped), so that two runs with the
+    same arguments save the same cells."""
+    total = int(np.prod(shape))
+    k = DUMP_PLANE_BYTES // itemsize
+    if total <= k:
+        return None
+    return np.unique(np.random.default_rng(seed).integers(0, total, size=k))
+
+
+def dump_outputs(torch, r, out_dir):
+    """Save what the step returned to its caller as out_dir/<name>.npy (float32 / float64): the per-band and
+    per-record arrays whole, the power and information planes whole or as the sample of plane_sample_index."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = plane_sample_index(r.power.shape, r.power.element_size())
+    arrays = {"frequency_hz": np.asarray(r.frequency_hz, dtype=np.float64), "band_power": r.band_power,
+              "total_power": r.total_power, "band_entropy_bits": r.band_entropy_bits, "entropy_bits": r.entropy_bits()}
+    if idx is None:
+        arrays["power"], arrays["info"] = r.power, r.info
+    else:
+        flat = torch.from_numpy(idx).to(r.power.device)
+        arrays["power"], arrays["info"] = r.power.reshape(-1)[flat], r.info.reshape(-1)[flat]
+    nbytes = 0
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        nbytes += a.nbytes
+    cells = int(np.prod(r.power.shape))
+    return {"dir": out_dir, "files": sorted(n + ".npy" for n in arrays), "bytes": nbytes,
+            "planes": "whole" if idx is None else
+                      f"{len(idx)} of {cells} cells of the flattened {list(r.power.shape)} plane, drawn with "
+                      "numpy default_rng(0) (bench.plane_sample_index)"}
+
+
 def timed_calls(torch, fn, reps, dist, dev):
     """Device time per call (ms), max over ranks, after one untimed call."""
     fn()
@@ -479,6 +520,8 @@ def run_gpu_arm(args):
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     elapsed_ms = float(t.item())
+    # before the end-to-end steps below write the same planes again
+    dumped = dump_outputs(torch, r, args.dump_outputs) if args.dump_outputs and rank == 0 else None
 
     # ---- end to end through the public API: pinned host records -> H2D -> kernels -> D2H of the summaries, K steps
     x_host = torch.empty(CH_PER_GPU, n, dtype=tdt, pin_memory=True)
@@ -584,6 +627,8 @@ def run_gpu_arm(args):
             "check": check,
             "configs": extras,
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         json_out.write(json.dumps(line) + "\n")
         json_out.flush()
     if dist is not None:
@@ -597,7 +642,14 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save what the last one computed as DIR/<name>.npy (rank 0's channels; "
+                         "the planes as a fixed sample, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs saves the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
