@@ -97,8 +97,42 @@ template <typename T, int DIR> QI_DEV void dit8(cplx<T>* a) {
     a[2] = b2 + b6; a[6] = b2 - b6; a[3] = b3 + b7; a[7] = b3 - b7;
 }
 
+// radix 16 = one radix-2 step around two radix-8 halves.  * w16^n for the odd n (n = 1, 3, 5, 7, sign by DIR):
+template <typename T, int DIR, int N> QI_DEV cplx<T> rot16(cplx<T> a) {
+    const T c = (T)0.92387953251128675613, s = (T)0.38268343236508977173;     // cos, sin (pi / 8)
+    const T wr = N == 1 ? c : (N == 3 ? s : (N == 5 ? -s : -c));
+    const T wi = N == 1 ? s : (N == 3 ? c : (N == 5 ? c : s));
+    return DIR == FFT_FWD ? mk<T>(a.re * wr + a.im * wi, a.im * wr - a.re * wi)
+                          : mk<T>(a.re * wr - a.im * wi, a.im * wr + a.re * wi);
+}
+// natural slots in, bit-reversed slots out: a[brev4(f)] = frequency f.  Slots 0..7 hold the even frequencies in brev3
+// order (brev4(2m) = brev3(m)), slots 8..15 the odd ones (brev4(2m + 1) = 8 + brev3(m)).
+template <typename T, int DIR> QI_DEV void dif16(cplx<T>* a) {
+    cplx<T> d[8];
+#pragma unroll
+    for (int n = 0; n < 8; ++n) { d[n] = a[n] - a[n + 8]; a[n] = a[n] + a[n + 8]; }
+    d[1] = rot16<T, DIR, 1>(d[1]); d[2] = rot45<T, DIR>(d[2]); d[3] = rot16<T, DIR, 3>(d[3]);
+    d[4] = rot90<T, DIR>(d[4]);
+    d[5] = rot16<T, DIR, 5>(d[5]); d[6] = rot135<T, DIR>(d[6]); d[7] = rot16<T, DIR, 7>(d[7]);
+    dif8<T, DIR>(a);
+    dif8<T, DIR>(d);
+#pragma unroll
+    for (int n = 0; n < 8; ++n) a[n + 8] = d[n];
+}
+// bit-reversed slots in, natural slots out (exact mirror of dif16)
+template <typename T, int DIR> QI_DEV void dit16(cplx<T>* a) {
+    dit8<T, DIR>(a);
+    dit8<T, DIR>(a + 8);
+    a[9] = rot16<T, DIR, 1>(a[9]); a[10] = rot45<T, DIR>(a[10]); a[11] = rot16<T, DIR, 3>(a[11]);
+    a[12] = rot90<T, DIR>(a[12]);
+    a[13] = rot16<T, DIR, 5>(a[13]); a[14] = rot135<T, DIR>(a[14]); a[15] = rot16<T, DIR, 7>(a[15]);
+#pragma unroll
+    for (int n = 0; n < 8; ++n) { const cplx<T> d = a[n] - a[n + 8]; a[n] = a[n] + a[n + 8]; a[n + 8] = d; }
+}
+
 QI_HD int brev3(int f) { return ((f & 1) << 2) | (f & 2) | ((f >> 2) & 1); }
 QI_HD int brev2(int f) { return ((f & 1) << 1) | ((f >> 1) & 1); }
+QI_HD int brev4(int f) { return (brev3(f & 7) << 1) | (f >> 3); }
 
 // ---------------------------------------------------------------- one radix-2^STEP stage on a tile
 // tile[r*TP + c], R = 2^logR rows, TC columns; tw[m] = exp(-2*pi*i*m/R), m in [0,R).

@@ -295,7 +295,8 @@ mr_table_kernel(const MrDevBand* __restrict__ bands, i64 n_points, int half_w_ca
     __syncthreads();
     tile_fft<float, FFT_FWD>(tile, tw, b.logF, 1, 2);
     const float inv = 1.0f / (float)F;
-    for (int p = threadIdx.x; p < F; p += blockDim.x) tables[b.table_off + p] = tile[p * 2] * inv;
+    for (int p = threadIdx.x; p < F; p += blockDim.x)       // 2048-point tables: the warp order of mr_level2k_kernel
+        tables[b.table_off + (F == L2K_F ? l2k_tab_slot(p) : p)] = tile[p * 2] * inv;
 }
 
 // ---------------------------------------------------------------- A: overlap-save level convolution (generic)
@@ -345,7 +346,7 @@ mr_level_kernel(const float* __restrict__ x, MrLevelGeom g, const MrDevBand* __r
         for (int idx = threadIdx.x; idx < F * TC; idx += blockDim.x) {
             const int c = idx & (TC - 1);
             const int r = idx >> logTC;
-            tile_y[r * TP + c] = tile_x[r * TP + c] * K[r];
+            tile_y[r * TP + c] = tile_x[r * TP + c] * K[F == L2K_F ? l2k_tab_slot(r) : r];
         }
         __syncthreads();
         tile_fft<float, FFT_INV>(tile_y, tw, g.logF, TC, TP);

@@ -1,23 +1,35 @@
 // qi_mr_level2k.cuh -- "A" of the multirate CWT (see qi_mr.cu): overlap-save convolution of one level signal with all
-// bands of that level, 2048-point blocks, written for the lowest instruction count per output sample.
+// bands of that level, 2048-point blocks, written for the fewest passes over shared memory per output sample (the
+// kernel is bound by the shared-memory / L1 data pipe, not by HBM).
 //
 //   * A CTA of 256 threads convolves PAIRS of consecutive blocks: the two blocks are the two complex columns of a
-//     float4 row, so every shared-memory access is one 128-bit instruction and every index / twiddle computation is
-//     shared by two transforms.  The tile is [2048 rows] x 16 B with one padding row per 8 rows
-//     (phys(r) = r + (r >> 3)): all four stage geometries and the staging pattern are bank-conflict free and every
-//     address is "one base register + immediate".
-//   * radix 8-8-8-4, one radix-8 butterfly (two columns) per thread and stage.  Forward = DIF (natural -> bit-reversed),
-//     inverse = DIT (bit-reversed -> natural), as everywhere in this library (qi_fft.cuh).
-//   * forward: the first stage reads the real level signal straight from HBM (coalesced), the last (radix-4) stage
-//     leaves the block spectra X in REGISTERS (rows 4g .. 4g+3 of thread g and g+256).
-//   * per band: the first inverse stage multiplies those registers with the band's kernel table (two 128-bit loads per
-//     four rows, L1/L2 resident) and runs its radix-4 butterfly before anything touches shared memory; the last
-//     inverse stage hands its natural-order outputs from registers to HBM (level 0: |.|^2 -> power plane; deeper
-//     levels: the decimated complex output w_b).  Two tile buffers alternate between bands -> 3 barriers per band.
+//     float4 tile row.  The radix-8 stages work on whole rows (one 128-bit access serves both transforms); the radix-16
+//     stages give each thread ONE column, with the two threads holding the same rows of blocks a and b in adjacent lanes
+//     (t = 2u + column): a lane pair touches one 16-byte row, so a half warp's 64-bit access is conflict free exactly
+//     when its 8 rows are, and both lanes of a pair read the same band-table lines.
+//   * 2048 = 8 * 16 * 16.  Forward = DIF (natural -> bit-reversed), inverse = DIT (bit-reversed -> natural), as
+//     everywhere in this library (qi_fft.cuh); dif16 / dit16 keep the fully bit-reversed spectrum, so the band tables of
+//     mr_table_kernel and the envelope fold see the same row order as a radix-2 transform (the tables are stored in the
+//     warp order of l2k_tab_slot so that their loads stay coalesced).
+//   * forward: radix-8 at B=2048 straight from HBM (real input) -> tile, radix-16 at B=256 through the tile, radix-16 at
+//     B=16 read from the tile: thread (u, column) keeps rows 16u .. 16u+15 of its block's spectrum X in REGISTERS.
+//   * per band (level 0, and every level of the complex-TFR mode): X * K and the radix-16 B=16 stage in registers ->
+//     tile, radix-16 at B=256 through the tile, radix-8 at B=2048 read from the tile; its natural-order outputs go from
+//     registers to HBM (level 0: |.|^2 -> power plane; deeper levels: the decimated complex output w_b).  Two tile
+//     buffers alternate between bands: 4 tile accesses and 2 barriers per band.
+//   * per band pair (envelope bands, levels >= 1): the 16 register rows fold into rows 8u .. 8u+7 of the 1024-point
+//     spectrum, whose radix-8 B=8 stage runs in registers -> tile, radix-16 at B=128, radix-8 at B=1024 read -> the
+//     demodulated envelope: also 4 accesses and 2 barriers.
 //     band_sum (optional) receives sum |y|^2 over the record's own samples: the exact band power at level 0, the raw
 //     sum that mr_total_kernel turns into the band-power estimate at deeper levels.
-//   * twiddles come from a per-stage table laid out [slot pair][j] (built once per call by mr_twiddle2k_kernel with
-//     the exact sincospi roots, copied to shared memory per CTA): 4 conflict-free 128-bit loads per butterfly.
+//   * twiddles come from per-stage tables laid out [slot pair][j] (built once per call by mr_twiddle2k_kernel with the
+//     exact sincospi roots, copied to shared memory per CTA): conflict-free 128-bit loads, one per two slots.  The
+//     B=2048 twiddles depend on the thread only and stay in registers for the whole kernel.
+//   * tile rows: the 2048-row tile pads one row per 16 (l2k_phys), the 1024-row envelope tiles one row per 8
+//     (l2k_physe).  Rows a half warp touches per access, l2k_phys: t + 256 i (8 consecutive t), 256G + j + 16 i (8
+//     consecutive j), 16u + i (8 consecutive u -> 17u + i, distinct mod 8); l2k_physe: 8u + i (9u + i), 128G + j + 8 i
+//     and j + 128 i (8 consecutive j): every stage is bank-conflict free and every address is "base register +
+//     immediate".
 #pragma once
 #include "qi_fft.cuh"
 #include "qi_mr_expand.cuh"
@@ -27,39 +39,57 @@ namespace qi {
 
 constexpr int L2K_LOGF = 11;
 constexpr int L2K_F = 1 << L2K_LOGF;
-constexpr int L2K_TILE = L2K_F + L2K_F / 8;          // padded rows per tile buffer
-// twiddle rows: 2048-point stages B=2048 (j<256), B=256 (j<32), B=32 (j<4); 1024-point stages of the envelope bands
-// B=1024 (j<128), B=128 (j<16), B=16 (j<2); then 16 rows holding the 64 demodulation phases exp(-2 pi i m / 64)
-constexpr int L2K_TW0 = 0, L2K_TW1 = 256, L2K_TW2 = 288;
-constexpr int L2K_TWE0 = 292, L2K_TWE1 = 420, L2K_TWE2 = 436;
-constexpr int L2K_TWJ = 438;
-constexpr int L2K_DEMOD = 4 * L2K_TWJ;               // float4 index of the demodulation table (16 float4 = 64 phases / 2 ... see kernel)
-constexpr int L2K_TW_TOTAL = 4 * L2K_TWJ + 32;       // float4 elements in the whole table
+QI_HD int l2k_phys(int r) { return r + (r >> 4); }   // padded row of a 2048-row tile
+QI_HD int l2k_physe(int r) { return r + (r >> 3); }  // padded row of a 1024-row envelope tile
+constexpr int L2K_TILE = L2K_F + L2K_F / 8;          // rows per tile buffer: two 1024-row envelope tiles (>= l2k_phys(F))
+// Band tables of 2048-point levels (mr_table_kernel) are stored in warp order: bit-reversed row r = 16u + 2m + e (group u
+// of a radix-16 thread, float4 m of its rows, half e) sits at complex slot 2 (128 (u >> 4) + 16 m + (u & 15)) + e.  The 16
+// groups of a warp then read float4 m of their rows from 256 consecutive bytes: 2 cache lines per load instruction
+// instead of 16 (the lane pair of a group reads the same float4).
+QI_HD int l2k_tab_slot(int r) {
+    const int u = r >> 4, m = (r >> 1) & 7;
+    return ((((u >> 4) << 7) | (m << 4) | (u & 15)) << 1) | (r & 1);
+}
+QI_HD int l2k_tab_group(int u) { return ((u >> 4) << 7) | (u & 15); }   // float4 index of (group u, m = 0)
+// twiddle tables, float4 entries [m][j]: (w_B^(j * brev(2m)), w_B^(j * brev(2m+1))), brev = brev3 for the radix-8 stages
+// (m < 4), brev4 for the radix-16 stages (m < 8).  The first L2K_TW_SMEM entries are copied to shared memory:
+//   B=1024 (radix 8, j < 128), then radix 16 with L2K_TW16J rows per m: B=256 (j < 16) and B=128 (rows 16 + j, j < 8),
+//   then 32 float4 holding the 64 demodulation phases exp(-2 pi i m / 64);
+// the B=2048 stage (radix 8, j < 256) follows and is read into registers from global memory.
+constexpr int L2K_TWE0 = 0;
+constexpr int L2K_TW16 = 4 * 128, L2K_TW16J = 24;
+constexpr int L2K_DEMOD = L2K_TW16 + 8 * L2K_TW16J;
+constexpr int L2K_TW_SMEM = L2K_DEMOD + 32;
+constexpr int L2K_TWA = L2K_TW_SMEM;
+constexpr int L2K_TW_TOTAL = L2K_TWA + 4 * 256;     // float4 elements in the whole table
 constexpr int L2K_MAXB = 64;                         // bands per level handled by this kernel
 constexpr int L2K_THREADS = 256;
-constexpr size_t L2K_SMEM = (size_t)(2 * L2K_TILE + L2K_TW_TOTAL) * 16 + (size_t)(L2K_THREADS / 32) * L2K_MAXB * 4;
+constexpr size_t L2K_SMEM = (size_t)(2 * L2K_TILE + L2K_TW_SMEM) * 16 + (size_t)(L2K_THREADS / 32) * L2K_MAXB * 4;
 
-// tw[m * L2K_TWJ + row] = ( w_B^(j * brev3(2m)), w_B^(j * brev3(2m+1)) ),  w_B = exp(-2 pi i / B)
 __global__ void mr_twiddle2k_kernel(float4* __restrict__ tw) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= L2K_TW_TOTAL) return;
-    if (idx >= L2K_DEMOD) {                                    // two consecutive phases per float4
+    if (idx >= L2K_DEMOD && idx < L2K_TW_SMEM) {               // two consecutive phases per float4
         const int m = 2 * (idx - L2K_DEMOD);
         const cplx<float> w0 = conj(unit_root<float>((unsigned long long)m, 6));
         const cplx<float> w1 = conj(unit_root<float>((unsigned long long)(m + 1), 6));
         tw[idx] = make_float4(w0.re, w0.im, w1.re, w1.im);
         return;
     }
-    const int m = idx / L2K_TWJ, row = idx % L2K_TWJ;
-    int logB, j;
-    if (row < L2K_TW1) { logB = 11; j = row; }
-    else if (row < L2K_TW2) { logB = 8; j = row - L2K_TW1; }
-    else if (row < L2K_TWE0) { logB = 5; j = row - L2K_TW2; }
-    else if (row < L2K_TWE1) { logB = 10; j = row - L2K_TWE0; }
-    else if (row < L2K_TWE2) { logB = 7; j = row - L2K_TWE1; }
-    else { logB = 4; j = row - L2K_TWE2; }
-    const cplx<float> w0 = conj(unit_root<float>((unsigned long long)(j * brev3(2 * m)), logB));
-    const cplx<float> w1 = conj(unit_root<float>((unsigned long long)(j * brev3(2 * m + 1)), logB));
+    int m, j, logB, f0, f1;
+    if (idx < L2K_TW16) {
+        m = idx / 128; j = idx % 128; logB = 10;
+    } else if (idx < L2K_DEMOD) {
+        const int row = (idx - L2K_TW16) % L2K_TW16J;
+        m = (idx - L2K_TW16) / L2K_TW16J;
+        logB = row < 16 ? 8 : 7; j = row < 16 ? row : row - 16;
+    } else {
+        m = (idx - L2K_TWA) / 256; j = (idx - L2K_TWA) % 256; logB = 11;
+    }
+    if (idx >= L2K_TW16 && idx < L2K_DEMOD) { f0 = brev4(2 * m); f1 = brev4(2 * m + 1); }
+    else { f0 = brev3(2 * m); f1 = brev3(2 * m + 1); }
+    const cplx<float> w0 = conj(unit_root<float>((unsigned long long)(j * f0), logB));
+    const cplx<float> w1 = conj(unit_root<float>((unsigned long long)(j * f1), logB));
     tw[idx] = make_float4(w0.re, w0.im, w1.re, w1.im);
 }
 
@@ -78,46 +108,57 @@ struct MrLevelGeom {
     int no_sums;            // edge source bands (indices >= n_bands): no row of their own in the sum arrays
 };
 
-// radix-8 stage on the two columns of a float4 tile; rows base + i*H live at tile[p0 + i*STRIDE]
+// one column of the tile: element p of column c of a float4 tile is col[2 p] with col = (float2*)tile + c
+QI_DEV cplx<float> l2k_ld(const float2* col, int p) { const float2 v = col[2 * p]; return mk<float>(v.x, v.y); }
+QI_DEV void l2k_st(float2* col, int p, cplx<float> v) { col[2 * p] = make_float2(v.re, v.im); }
+
+// radix-16 stage on one column; rows base + i*H live at col[2 (p0 + i*STRIDE)], twiddles tw[L2K_TW16 + m L2K_TW16J + twrow]
 template <int DIR, int STRIDE>
-QI_DEV void l2k_stage8(float4* __restrict__ tile, int p0, const float4* __restrict__ tw, int twrow) {
-    cplx<float> a[8], b[8];
-    float4 w[4];
-#pragma unroll
-    for (int m = 0; m < 4; ++m) w[m] = tw[m * L2K_TWJ + twrow];
+QI_DEV void l2k_stage16(float2* __restrict__ col, int p0, const float4* __restrict__ tw, int twrow) {
+    cplx<float> a[16];
+    const float4* w = tw + L2K_TW16 + twrow;
     if (DIR == FFT_FWD) {
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float4 v = tile[p0 + i * STRIDE];
-            a[i] = mk<float>(v.x, v.y); b[i] = mk<float>(v.z, v.w);
-        }
-        dif8<float, DIR>(a); dif8<float, DIR>(b);
+        for (int i = 0; i < 16; ++i) a[i] = l2k_ld(col, p0 + i * STRIDE);
+        dif16<float, DIR>(a);
 #pragma unroll
-        for (int s = 0; s < 8; ++s) {
-            cplx<float> va = a[s], vb = b[s];
-            if (s) {
-                const float4 ww = w[s >> 1];
-                const cplx<float> t = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                va = va * t; vb = vb * t;
-            }
-            tile[p0 + s * STRIDE] = make_float4(va.re, va.im, vb.re, vb.im);
+        for (int m = 0; m < 8; ++m) {
+            cplx<float> v0 = a[2 * m], v1 = a[2 * m + 1];
+            const float4 ww = w[m * L2K_TW16J];
+            if (m) v0 = v0 * mk<float>(ww.x, ww.y);
+            v1 = v1 * mk<float>(ww.z, ww.w);
+            l2k_st(col, p0 + 2 * m * STRIDE, v0);
+            l2k_st(col, p0 + (2 * m + 1) * STRIDE, v1);
         }
     } else {
 #pragma unroll
-        for (int s = 0; s < 8; ++s) {
-            const float4 v = tile[p0 + s * STRIDE];
-            cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
-            if (s) {
-                const float4 ww = w[s >> 1];
-                const cplx<float> t = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                va = mul_conj(va, t); vb = mul_conj(vb, t);
-            }
-            a[s] = va; b[s] = vb;
+        for (int m = 0; m < 8; ++m) {
+            const float4 ww = w[m * L2K_TW16J];
+            a[2 * m] = l2k_ld(col, p0 + 2 * m * STRIDE);
+            a[2 * m + 1] = mul_conj(l2k_ld(col, p0 + (2 * m + 1) * STRIDE), mk<float>(ww.z, ww.w));
+            if (m) a[2 * m] = mul_conj(a[2 * m], mk<float>(ww.x, ww.y));
         }
-        dit8<float, DIR>(a); dit8<float, DIR>(b);
+        dit16<float, DIR>(a);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) tile[p0 + i * STRIDE] = make_float4(a[i].re, a[i].im, b[i].re, b[i].im);
+        for (int i = 0; i < 16; ++i) l2k_st(col, p0 + i * STRIDE, a[i]);
     }
+}
+
+// radix-8 DIT stage on both columns of a float4 tile, rows base + s*H at tile[p0 + s*STRIDE], per-thread twiddles w
+QI_DEV void l2k_read_dit8(const float4* __restrict__ tile, int p0, int stride, const float4 (&w)[4], cplx<float> (&a)[8],
+                          cplx<float> (&c)[8]) {
+#pragma unroll
+    for (int s = 0; s < 8; ++s) {
+        const float4 v = tile[p0 + s * stride];
+        cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
+        if (s) {
+            const float4 ww = w[s >> 1];
+            const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
+            va = mul_conj(va, tt); vb = mul_conj(vb, tt);
+        }
+        a[s] = va; c[s] = vb;
+    }
+    dit8<float, FFT_INV>(a); dit8<float, FFT_INV>(c);
 }
 
 // bx: index of this CTA among the CTAs of its level (blockIdx.x, or the offset inside a merged multi-level launch)
@@ -131,7 +172,7 @@ QI_DEV void l2k_body(const float* __restrict__ x, const MrLevelGeom& g, const Mr
     float4* tile0 = reinterpret_cast<float4*>(smem_raw);
     float4* tile1 = tile0 + L2K_TILE;
     float4* tw = tile1 + L2K_TILE;
-    float* wsum = reinterpret_cast<float*>(tw + L2K_TW_TOTAL);         // [warps][L2K_MAXB]
+    float* wsum = reinterpret_cast<float*>(tw + L2K_TW_SMEM);          // [warps][L2K_MAXB]
     const int t = threadIdx.x;
     const int warp = t >> 5, lane = t & 31;
     const i64 chan = blockIdx.y;
@@ -139,23 +180,19 @@ QI_DEV void l2k_body(const float* __restrict__ x, const MrLevelGeom& g, const Mr
     const int half = g.wk / 2;
     const float* xs = x + chan * g.x_stride;
 
-    for (int i = t; i < L2K_TW_TOTAL; i += L2K_THREADS) tw[i] = tw_g[i];
+    for (int i = t; i < L2K_TW_SMEM; i += L2K_THREADS) tw[i] = tw_g[i];
     for (int i = t; i < (L2K_THREADS / 32) * L2K_MAXB; i += L2K_THREADS) wsum[i] = 0.0f;
 
     // per-thread tile addresses (padded rows), fixed for the whole kernel
-    const int pA = t + (t >> 3);                                           // stage B=2048: rows t + 256 i   -> + 288 i
-    const int rB = ((t >> 5) << 8) + (t & 31);                             // stage B=256 : rows rB + 32 i   -> + 36 i
-    const int pB = rB + (rB >> 3);
-    const int pC = (t >> 2) * 36 + (t & 3);                                // stage B=32  : rows 32G + j + 4i -> + 4i + (i>>1)
-    const int pD0 = 4 * t + (t >> 1);                                      // radix 4     : rows 4g + i, g = t
-    const int pD1 = 4 * (t + 256) + ((t + 256) >> 1);                      //               g = t + 256
+    const int pA = l2k_phys(t);                                            // B=2048: rows t + 256 i    -> + 272 i
+    const int cl = t & 1, u = t >> 1;                                      // radix-16 stages: column, row group
+    const int pB = 272 * (u >> 4) + (u & 15);                              // B=256 : rows 256G + j + 16 i -> + 17 i
+    const int pC = 17 * u;                                                 // B=16  : rows 16u + i         -> + i
 
     // twiddles of the stage B=2048 depend on the thread only: kept in registers for the forward stage and every band
-    // (the kernel is bound by the shared-memory / L1 data pipe: 73 % of its wavefront rate, ncu r3c)
-    __syncthreads();
     float4 wA[4];
 #pragma unroll
-    for (int m = 0; m < 4; ++m) wA[m] = tw[m * L2K_TWJ + L2K_TW0 + t];
+    for (int m = 0; m < 4; ++m) wA[m] = tw_g[L2K_TWA + m * 256 + t];
 
     for (int pp = 0; pp < pairs_per_cta; ++pp) {
         const i64 blk0 = 2 * ((i64)bx * pairs_per_cta + pp);
@@ -181,123 +218,58 @@ QI_DEV void l2k_body(const float* __restrict__ x, const MrLevelGeom& g, const Mr
                     const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
                     va = va * tt; vb = vb * tt;
                 }
-                tile0[pA + s * 288] = make_float4(va.re, va.im, vb.re, vb.im);
+                tile0[pA + s * 272] = make_float4(va.re, va.im, vb.re, vb.im);
             }
         }
         __syncthreads();
-        l2k_stage8<FFT_FWD, 36>(tile0, pB, tw, L2K_TW1 + (t & 31));
+        l2k_stage16<FFT_FWD, 17>(reinterpret_cast<float2*>(tile0) + cl, pB, tw, u & 15);
         __syncthreads();
-        {   // stage B=32: rows 32G + j + 4i -> pC + 4i + (i >> 1): not a constant stride, spelled out
-            cplx<float> a[8], b[8];
-            float4 w[4];
+        // ---- forward stage B=16: the spectrum of block cl stays in registers (bit-reversed rows 16u .. 16u+15)
+        cplx<float> X[16];
+        {
+            const float2* col = reinterpret_cast<const float2*>(tile0) + cl;
 #pragma unroll
-            for (int m = 0; m < 4; ++m) w[m] = tw[m * L2K_TWJ + L2K_TW2 + (t & 3)];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const float4 v = tile0[pC + 4 * i + (i >> 1)];
-                a[i] = mk<float>(v.x, v.y); b[i] = mk<float>(v.z, v.w);
-            }
-            dif8<float, FFT_FWD>(a); dif8<float, FFT_FWD>(b);
-#pragma unroll
-            for (int s = 0; s < 8; ++s) {
-                cplx<float> va = a[s], vb = b[s];
-                if (s) {
-                    const float4 ww = w[s >> 1];
-                    const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                    va = va * tt; vb = vb * tt;
-                }
-                tile0[pC + 4 * s + (s >> 1)] = make_float4(va.re, va.im, vb.re, vb.im);
-            }
-        }
-        __syncthreads();
-        // ---- forward radix-4 stage: spectra stay in registers (rows 4g .. 4g+3, g = t and t + 256)
-        cplx<float> X0[2][4], X1[2][4];
-#pragma unroll
-        for (int task = 0; task < 2; ++task) {
-            const int p = task ? pD1 : pD0;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float4 v = tile0[p + i];
-                X0[task][i] = mk<float>(v.x, v.y); X1[task][i] = mk<float>(v.z, v.w);
-            }
-            dif4<float, FFT_FWD>(X0[task]); dif4<float, FFT_FWD>(X1[task]);
+            for (int i = 0; i < 16; ++i) X[i] = l2k_ld(col, pC + i);
+            dif16<float, FFT_FWD>(X);
         }
 
         // ---- envelope bands: two bands per pass, half-size inverse transforms (see mr_plan)
         //   fold   Z[k'] = Y[k'] + Y[k' + 1024]  <->  rows (2q, 2q+1) of the bit-reversed 2048-row spectrum add up to
         //          row q of the bit-reversed 1024-row one: y(2m) = IFFT_1024(Z)(m)
-        //   the first (radix-2) stage of that transform joins rows (2g, 2g+1): still inside the thread that holds rows
-        //   4g .. 4g+3 of Y; then radix 8-8-8 with 128 butterflies per band, i.e. 256 = both bands of the pass
+        //   rows 16u .. 16u+15 of Y fold into rows 8u .. 8u+7 of Z, whose radix-8 B=8 stage runs in registers; then
+        //   radix-16 at B=128 (64 butterflies per band and column) and radix-8 at B=1024 (128 per band, both columns)
         for (int pi = 0; ENV && g.env && pi < g.band_count; pi += 2) {
             const int nbp = g.band_count - pi < 2 ? g.band_count - pi : 2;
             float4* tile = ((pi >> 1) & 1) ? tile0 : tile1;
+            for (int bb = 0; bb < nbp; ++bb) {
+                const float4* K = reinterpret_cast<const float4*>(tables + bands[g.band_first + pi + bb].table_off) +
+                                 l2k_tab_group(u);
+                cplx<float> z[8];
 #pragma unroll
-            for (int task = 0; task < 2; ++task) {
-                const int gq = t + 256 * task;
-                const int p = 2 * gq + (gq >> 2);                          // padded row of 2 gq in a 1024-row tile
-                for (int bb = 0; bb < nbp; ++bb) {
-                    const float4* K = reinterpret_cast<const float4*>(tables + bands[g.band_first + pi + bb].table_off);
-                    const float4 k01 = K[2 * gq], k23 = K[2 * gq + 1];
-                    const cplx<float> kk[4] = {mk<float>(k01.x, k01.y), mk<float>(k01.z, k01.w), mk<float>(k23.x, k23.y),
-                                               mk<float>(k23.z, k23.w)};
-                    const cplx<float> za0 = X0[task][0] * kk[0] + X0[task][1] * kk[1];
-                    const cplx<float> za1 = X0[task][2] * kk[2] + X0[task][3] * kk[3];
-                    const cplx<float> zc0 = X1[task][0] * kk[0] + X1[task][1] * kk[1];
-                    const cplx<float> zc1 = X1[task][2] * kk[2] + X1[task][3] * kk[3];
-                    const cplx<float> a0 = za0 + za1, a1 = za0 - za1, c0 = zc0 + zc1, c1 = zc0 - zc1;
-                    tile[bb * (L2K_TILE / 2) + p] = make_float4(a0.re, a0.im, c0.re, c0.im);
-                    tile[bb * (L2K_TILE / 2) + p + 1] = make_float4(a1.re, a1.im, c1.re, c1.im);
+                for (int m = 0; m < 8; ++m) {
+                    const float4 k = K[16 * m];
+                    z[m] = X[2 * m] * mk<float>(k.x, k.y) + X[2 * m + 1] * mk<float>(k.z, k.w);
                 }
+                dit8<float, FFT_INV>(z);
+                float2* col = reinterpret_cast<float2*>(tile + bb * (L2K_TILE / 2)) + cl;
+#pragma unroll
+                for (int i = 0; i < 8; ++i) l2k_st(col, 9 * u + i, z[i]);         // l2k_physe(8u + i)
             }
             __syncthreads();
-            const int bb = t >> 7, u = t & 127;                            // band of the pass / butterfly of that band
-            const bool live = bb < nbp;
-            float4* tb = tile + bb * (L2K_TILE / 2);
-            if (live) {   // stage B=16: rows 16G + j + 2i -> 18G + j + 2i + (i >> 2)
-                const int p0 = (u >> 1) * 18 + (u & 1);
+            {   // stage B=128: rows 128G + j + 8i -> 144G + j + 9i, band u >> 6 of the pass
+                const int bb = u >> 6, G = (u >> 3) & 7, j = u & 7;
+                if (bb < nbp)
+                    l2k_stage16<FFT_INV, 9>(reinterpret_cast<float2*>(tile + bb * (L2K_TILE / 2)) + cl, 144 * G + j, tw,
+                                            16 + j);
+            }
+            __syncthreads();
+            const int bb = t >> 7, v = t & 127;                            // band of the pass / butterfly of that band
+            if (bb < nbp) {   // stage B=1024: rows v + 128i -> v + (v >> 3) + 144i; outputs m = v + 128 i leave from registers
                 cplx<float> a[8], c[8];
                 float4 w[4];
 #pragma unroll
-                for (int m = 0; m < 4; ++m) w[m] = tw[m * L2K_TWJ + L2K_TWE2 + (u & 1)];
-#pragma unroll
-                for (int s = 0; s < 8; ++s) {
-                    const float4 v = tb[p0 + 2 * s + (s >> 2)];
-                    cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
-                    if (s) {
-                        const float4 ww = w[s >> 1];
-                        const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                        va = mul_conj(va, tt); vb = mul_conj(vb, tt);
-                    }
-                    a[s] = va; c[s] = vb;
-                }
-                dit8<float, FFT_INV>(a); dit8<float, FFT_INV>(c);
-#pragma unroll
-                for (int i = 0; i < 8; ++i) tb[p0 + 2 * i + (i >> 2)] = make_float4(a[i].re, a[i].im, c[i].re, c[i].im);
-            }
-            __syncthreads();
-            if (live) {   // stage B=128: rows 128G + j + 16i -> 144G + j + (j >> 3) + 18i
-                const int j = u & 15;
-                l2k_stage8<FFT_INV, 18>(tb, (u >> 4) * 144 + j + (j >> 3), tw, L2K_TWE1 + j);
-            }
-            __syncthreads();
-            if (live) {   // stage B=1024: rows j + 128i -> j + (j >> 3) + 144i; outputs m = u + 128 i leave from registers
-                cplx<float> a[8], c[8];
-                float4 w[4];
-#pragma unroll
-                for (int m = 0; m < 4; ++m) w[m] = tw[m * L2K_TWJ + L2K_TWE0 + u];
-                const int p0 = u + (u >> 3);
-#pragma unroll
-                for (int s = 0; s < 8; ++s) {
-                    const float4 v = tb[p0 + 144 * s];
-                    cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
-                    if (s) {
-                        const float4 ww = w[s >> 1];
-                        const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                        va = mul_conj(va, tt); vb = mul_conj(vb, tt);
-                    }
-                    a[s] = va; c[s] = vb;
-                }
-                dit8<float, FFT_INV>(a); dit8<float, FFT_INV>(c);
+                for (int m = 0; m < 4; ++m) w[m] = tw[L2K_TWE0 + m * 128 + v];
+                l2k_read_dit8(tile + bb * (L2K_TILE / 2), l2k_physe(v), 144, w, a, c);
                 const int b = g.band_first + pi + bb;
                 const MrDevBand band = bands[b];
                 const cplx<float>* dm = reinterpret_cast<const cplx<float>*>(tw + L2K_DEMOD);   // exp(-2 pi i m / 64)
@@ -312,7 +284,7 @@ QI_DEV void l2k_body(const float* __restrict__ x, const MrLevelGeom& g, const Mr
                     cplx<float>* wdst = wbuf + band.w_off + chan * band.w_stride;
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        const int mm = u + 128 * i - hh;
+                        const int mm = v + 128 * i - hh;
                         const i64 wi = blk * Vh + mm;                       // index into w (halo included): q' = wi - HALO
                         if (mm >= 0 && mm < Vh && wi < n_w) {
                             const i64 q = wi - MR_HALO;
@@ -333,63 +305,27 @@ QI_DEV void l2k_body(const float* __restrict__ x, const MrLevelGeom& g, const Mr
         for (int bi = 0; !(ENV && g.env) && bi < g.band_count; ++bi) {
             const int b = g.band_first + bi;
             const MrDevBand band = bands[b];
-            const float4* K = reinterpret_cast<const float4*>(tables + band.table_off);
             float4* tile = (bi & 1) ? tile0 : tile1;
-            // inverse radix-4 stage on X * K, from registers
+            {   // inverse stage B=16 on X * K, from registers
+                const float4* K = reinterpret_cast<const float4*>(tables + band.table_off) + l2k_tab_group(u);
+                cplx<float> a[16];
 #pragma unroll
-            for (int task = 0; task < 2; ++task) {
-                const int gq = t + 256 * task;
-                const float4 k01 = K[2 * gq], k23 = K[2 * gq + 1];
-                const cplx<float> kk[4] = {mk<float>(k01.x, k01.y), mk<float>(k01.z, k01.w), mk<float>(k23.x, k23.y),
-                                           mk<float>(k23.z, k23.w)};
-                cplx<float> a[4], c[4];
-#pragma unroll
-                for (int s = 0; s < 4; ++s) { a[s] = X0[task][s] * kk[s]; c[s] = X1[task][s] * kk[s]; }
-                dit4<float, FFT_INV>(a); dit4<float, FFT_INV>(c);
-                const int p = task ? pD1 : pD0;
-#pragma unroll
-                for (int i = 0; i < 4; ++i) tile[p + i] = make_float4(a[i].re, a[i].im, c[i].re, c[i].im);
-            }
-            __syncthreads();
-            {   // stage B=32
-                cplx<float> a[8], c[8];
-                float4 w[4];
-#pragma unroll
-                for (int m = 0; m < 4; ++m) w[m] = tw[m * L2K_TWJ + L2K_TW2 + (t & 3)];
-#pragma unroll
-                for (int s = 0; s < 8; ++s) {
-                    const float4 v = tile[pC + 4 * s + (s >> 1)];
-                    cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
-                    if (s) {
-                        const float4 ww = w[s >> 1];
-                        const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                        va = mul_conj(va, tt); vb = mul_conj(vb, tt);
-                    }
-                    a[s] = va; c[s] = vb;
+                for (int m = 0; m < 8; ++m) {
+                    const float4 k = K[16 * m];
+                    a[2 * m] = X[2 * m] * mk<float>(k.x, k.y);
+                    a[2 * m + 1] = X[2 * m + 1] * mk<float>(k.z, k.w);
                 }
-                dit8<float, FFT_INV>(a); dit8<float, FFT_INV>(c);
+                dit16<float, FFT_INV>(a);
+                float2* col = reinterpret_cast<float2*>(tile) + cl;
 #pragma unroll
-                for (int i = 0; i < 8; ++i) tile[pC + 4 * i + (i >> 1)] = make_float4(a[i].re, a[i].im, c[i].re, c[i].im);
+                for (int i = 0; i < 16; ++i) l2k_st(col, pC + i, a[i]);
             }
             __syncthreads();
-            l2k_stage8<FFT_INV, 36>(tile, pB, tw, L2K_TW1 + (t & 31));
+            l2k_stage16<FFT_INV, 17>(reinterpret_cast<float2*>(tile) + cl, pB, tw, u & 15);
             __syncthreads();
             // ---- last stage B=2048: outputs n = t + 256 i leave from registers
             cplx<float> a[8], c[8];
-            {
-#pragma unroll
-                for (int s = 0; s < 8; ++s) {
-                    const float4 v = tile[pA + s * 288];
-                    cplx<float> va = mk<float>(v.x, v.y), vb = mk<float>(v.z, v.w);
-                    if (s) {
-                        const float4 ww = wA[s >> 1];
-                        const cplx<float> tt = (s & 1) ? mk<float>(ww.z, ww.w) : mk<float>(ww.x, ww.y);
-                        va = mul_conj(va, tt); vb = mul_conj(vb, tt);
-                    }
-                    a[s] = va; c[s] = vb;
-                }
-                dit8<float, FFT_INV>(a); dit8<float, FFT_INV>(c);
-            }
+            l2k_read_dit8(tile, pA, 272, wA, a, c);
             float acc = 0.0f;
 #pragma unroll
             for (int col = 0; col < 2; ++col) {
