@@ -130,8 +130,10 @@ typedef struct {
 
 size_t qi_cwt_multirate_workspace_bytes(int64_t n_channels, int64_t n_points, const QiMrBand* bands, int n_bands);
 
-/* out_power float [C,B,N] or NULL; out_cwt complex64 [C,B,N] or NULL; band_sum double [C,B] (exact sums of the
- * stored power) or NULL.
+/* sig float [C, sig_stride]: 16-byte aligned, sig_stride a multiple of 4 samples (the record is read with 128-bit
+ * loads); a record that starts elsewhere, such as a slice x[k:] of a device buffer, is QI_ERR_ARG, so copy it first.
+ * out_power float [C,B,N] or NULL; out_cwt complex64 [C,B,N] or NULL; band_sum double [C,B] (exact sums of the
+ * stored power) or NULL; out_power, out_cwt and out_info 32-byte aligned.
  *
  * Fused information / entropy (replaces tfr_info.py:231-236 on top of the CWT, one pass over the planes):
  * pass out_info float [C,B,N]; then out_power, band_sum, band_sum_est [C,B] and total_power [C] are required and

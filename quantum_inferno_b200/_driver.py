@@ -299,6 +299,11 @@ def cwt_multirate(sig, bands, want_power=True, want_complex=False, want_band_sum
     rt = rt or get_runtime()
     lib = rt.lib
     C, N = int(sig.shape[0]), int(sig.shape[1])
+    if rt.ptr(sig) % 16:
+        # the kernels read the record as float4; a slice x[k:] of a device buffer can start anywhere on a 4-byte grid
+        buf = rt.empty((C, N), "float32")
+        buf[...] = sig
+        sig = buf
     bands = np.ascontiguousarray(bands, dtype=_lib.MR_BAND)
     B = len(bands)
     nbytes = lib.qi_cwt_multirate_workspace_bytes(C, N, bands.ctypes.data, B)

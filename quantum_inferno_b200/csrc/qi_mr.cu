@@ -858,8 +858,9 @@ int qi_cwt_multirate(const void* sig, int64_t C, int64_t N, int64_t stride, cons
                      double* band_sum_est, double* total_power, double eps, int phase, void* ws, size_t ws_bytes,
                      void* stream) {
     if (!sig || !bands || !ws || C <= 0 || N <= 0 || B <= 0 || stride < N) return QI_ERR_ARG;
-    // vector loads / 256-bit plane stores: records 8-byte aligned with an even stride, planes 32-byte aligned
-    if (((uintptr_t)sig & 7) || (stride & 1) || ((uintptr_t)out_power & 31) || ((uintptr_t)out_info & 31) ||
+    // vector loads / 256-bit plane stores: records 16-byte aligned with a stride that is a multiple of 4 samples (the
+    // edge rows read the record as float4 in mr_expand_kernel), planes 32-byte aligned
+    if (((uintptr_t)sig & 15) || (stride & 3) || ((uintptr_t)out_power & 31) || ((uintptr_t)out_info & 31) ||
         ((uintptr_t)out_complex & 31))
         return QI_ERR_ARG;
     if (!out_power && !out_complex && !band_sum) return QI_ERR_ARG;

@@ -1,7 +1,7 @@
 """
-CPU tier: the kernel sources, compiled for the CPU emulator with AddressSanitizer, run every kernel family once
-(tests/emul/asan_check.sh + asan_driver.py).  compute-sanitizer is closed on the GPU pool; an out-of-bounds access to a
-global buffer or to shared memory shows up here instead.  Test infrastructure only -- the package never loads the emulator.
+CPU tier: the kernel sources, compiled for the CPU emulator with AddressSanitizer and -fsanitize=alignment, run every
+kernel family once (tests/emul/asan_check.sh + asan_driver.py).  compute-sanitizer is closed on the GPU pool; an
+out-of-bounds access to a global buffer or to shared memory, or a misaligned vector access, shows up here instead.  Test infrastructure only -- the package never loads the emulator.
 """
 import os
 import shutil
@@ -24,4 +24,5 @@ def test_kernels_under_address_sanitizer(tmp_path):
     tail = (run.stdout + run.stderr)[-3000:]
     assert run.returncode == 0, tail
     assert "AddressSanitizer" not in run.stdout + run.stderr, tail
+    assert "runtime error:" not in run.stdout + run.stderr, tail        # -fsanitize=alignment: misaligned vector access
     assert "asan run done" in run.stdout, tail
