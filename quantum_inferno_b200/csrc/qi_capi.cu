@@ -80,20 +80,13 @@ template <typename T>
 static int fft_c2c_impl(const void* in, void* out, i64 batch, int log2n, int inverse, cudaStream_t st) {
     const FftPlan plan = make_plan(log2n, (int)sizeof(cplx<T>));
     const i64 n = 1ll << log2n;
-    const cplx<T>* src0 = static_cast<const cplx<T>*>(in);
+    const SrcComplex<T> src{static_cast<const cplx<T>*>(in), n};
     cplx<T>* dstp = static_cast<cplx<T>*>(out);
     if (!inverse) {
-        for (int p = 0; p < plan.npass; ++p) {
-            SrcComplex<T> s{p == 0 ? src0 : dstp, n};
-            DstComplex<T> d{dstp, n, (T)1};
-            launch_pass<T, FFT_FWD>(plan, p, batch, s, d, 0, st);
-        }
+        forward_passes<T>(plan, batch, src, dstp, n, st);
     } else {
-        for (int p = plan.npass - 1; p >= 0; --p) {
-            SrcComplex<T> s{p == plan.npass - 1 ? src0 : dstp, n};
-            DstComplex<T> d{dstp, n, p == 0 ? (T)(1.0 / (double)n) : (T)1};
-            launch_pass<T, FFT_INV>(plan, p, batch, s, d, 0, st);
-        }
+        inverse_passes<T>(plan, batch, src, DstComplex<T>{dstp, n, (T)(1.0 / (double)n)}, 0, false, dstp, n, st);
+        prof_set_category(QI_CAT_OTHER);
     }
     return check_cuda("qi_fft_c2c");
 }
@@ -117,16 +110,7 @@ static int rfft_impl(const void* sig, i64 M, i64 n, i64 stride, void* out, void*
     if (M > 65535) return QI_ERR_UNSUPPORTED;
     cplx<T>* spec = static_cast<cplx<T>*>(ws);
     const FftPlan plan = make_plan(logn, (int)sizeof(cplx<T>));
-    for (int p = 0; p < plan.npass; ++p) {
-        DstComplex<T> d{spec, n, (T)1};
-        if (p == 0) {
-            SrcRealPad<T> s{static_cast<const T*>(sig), stride, n};
-            launch_pass<T, FFT_FWD>(plan, p, M, s, d, 0, st);
-        } else {
-            SrcComplex<T> s{spec, n};
-            launch_pass<T, FFT_FWD>(plan, p, M, s, d, 0, st);
-        }
-    }
+    forward_passes<T>(plan, M, SrcRealPad<T>{static_cast<const T*>(sig), stride, n}, spec, n, st);
     dim3 grid((unsigned)((n / 2 + 1 + 255) / 256), (unsigned)M);
     QI_LAUNCH((half_spectrum_gather_kernel<T>), grid, dim3(256), 0, st, (const cplx<T>*)spec, logn, static_cast<cplx<T>*>(out));
     return check_cuda("qi_rfft");

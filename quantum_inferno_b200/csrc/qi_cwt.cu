@@ -243,8 +243,6 @@ static int cwt_fft_impl(const void* sig, i64 C, i64 N, i64 stride, const QiAtomB
     geo.d_max = N - 1 - geo.centre_idx;
 
     const FftPlan plan = make_plan(lo.logL, (int)sizeof(cplx<T>));
-    const int np = plan.npass;
-    const T one = (T)1;
     if (band_sum) cudaMemsetAsync(band_sum, 0, sizeof(double) * (size_t)C * B, st);
 
     // ---- (S) short atoms: overlap-save in shared memory, straight from the record
@@ -262,109 +260,32 @@ static int cwt_fft_impl(const void* sig, i64 C, i64 N, i64 stride, const QiAtomB
         prof_set_category(QI_CAT_FFT_FWD);
         QI_LAUNCH((cwtf_os_table_kernel<T>), dim3((unsigned)((1 << logF) / 256), (unsigned)n_os), dim3(256), 0, st,
                   (const DevBand*)d_bandsF, logF, half_shift, tabF);
-        const int V = (1 << logF) - 2 * fp.os_half;
-        const size_t smem = sizeof(cplx<T>) * (2 * (size_t)pad8(1 << logF) + ((size_t)1 << logF)) + 256;
-#ifndef QI_EMUL
-        cudaFuncSetAttribute(cwtf_os_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-#endif
-        prof_set_category(QI_CAT_INV_LAST);
-        QI_LAUNCH((cwtf_os_kernel<T>), dim3((unsigned)((N + V - 1) / V), (unsigned)C), dim3(512), smem, st,
-                  static_cast<const T*>(sig), stride, geo, (const int*)d_os, n_os, logF, fp.os_half, (const cplx<T>*)tabF,
-                  static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum);
+        overlap_save_route<T>(sig, stride, geo, d_os, n_os, fp.os_half, OsTableRoute<T>{tabF}, out_c, out_p, band_sum, st);
     }
 
     // record spectra (the overlap-save route does not need them)
-    if (fp.n_plain > 0 || !fp.dec_ids.empty()) {
-        prof_set_category(QI_CAT_FFT_FWD);
-        for (int p = 0; p < np; ++p) {
-            DstComplex<T> d{spec, lo.L, one};
-            if (p == 0) {
-                SrcRealPad<T> s{static_cast<const T*>(sig), stride, N};
-                launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st);
-            } else {
-                SrcComplex<T> s{spec, lo.L};
-                launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st);
-            }
-        }
-    }
+    prof_set_category(QI_CAT_FFT_FWD);
+    if ((int)fp.os_ids.size() < B)
+        forward_passes<T>(plan, C, SrcRealPad<T>{static_cast<const T*>(sig), stride, N}, spec, lo.L, st);
     // atom tables (one forward FFT per table band, shared by all channels)
-    if (n_tab) {
-        for (int p = 0; p < np; ++p) {
-            DstComplex<T> d{tables, lo.L, one};
-            if (p == 0) {
-                SrcAtomKernel<T> s{d_bands, d_tab, geo};
-                launch_pass<T, FFT_FWD>(plan, p, n_tab, s, d, 0, st);
-            } else {
-                SrcComplex<T> s{tables, lo.L};
-                launch_pass<T, FFT_FWD>(plan, p, n_tab, s, d, 0, st);
-            }
-        }
-    }
+    if (n_tab) forward_passes<T>(plan, n_tab, SrcAtomKernel<T>{d_bands, d_tab, geo}, tables, lo.L, st);
 
     // ---- (D) long decayed atoms: baseband bins -> short inverse transform -> Kaiser-sinc interpolation
-    if (!fp.dec_ids.empty()) {
-        typedef CwtFastCfg<T> Cfg;
-        int* d_dec = reinterpret_cast<int*>(base + lo.off_ids) + B;
-        T* coef = reinterpret_cast<T*>(base + lo.off_coef);
-        stage_to_device(d_dec, fp.dec_ids.data(), sizeof(int) * fp.dec_ids.size(), st);
-        unsigned need_mask = 0;
-        for (int b : fp.dec_ids) need_mask |= 1u << (lo.logL - fp.logK[b]);
-        prof_set_category(QI_CAT_OTHER);
-        QI_LAUNCH((cwtf_coef_kernel<T>), dim3((unsigned)((Cfg::TAPS << CWTF_MAX_LOGD) / 256 + 1), (unsigned)(CWTF_MAX_LOGD + 1)),
-                  dim3(256), 0, st, coef, need_mask, 1.0 / cwtf_bessel_i0(Cfg::BETA));
-        const size_t work_elems = (size_t)lo.group * C * lo.L;
-        size_t pos = 0;
-        while (pos < fp.dec_ids.size()) {
-            const int lk = fp.logK[fp.dec_ids[pos]];
-            size_t end = pos;
-            while (end < fp.dec_ids.size() && fp.logK[fp.dec_ids[end]] == lk) ++end;
-            const int logD = lo.logL - lk;
-            const T* cf = coef + (size_t)logD * Cfg::TAPS * (1u << CWTF_MAX_LOGD);
-            const FftPlan pk = make_plan(lk, (int)sizeof(cplx<T>));
-            const i64 K = 1ll << lk;
-            for (size_t sub = pos; sub < end;) {
-                i64 gs = (i64)(end - sub);
-                while (gs * C > 65535 || (size_t)gs * C * K > work_elems) --gs;
-                if (gs < 1) return QI_ERR_WORKSPACE;
-                const i64 nb = gs * C;
-                SrcCwtDec<T> s1{spec, d_bands, d_dec + sub, (int)C, lo.logL, lk, half_shift};
-                for (int p = pk.npass - 1; p >= 0; --p) {
-                    const bool first = (p == pk.npass - 1);
-                    SrcComplex<T> s2{work, K};
-                    DstComplex<T> dw{work, K, one};
-                    prof_set_category(first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID);
-                    if (first) launch_pass<T, FFT_INV>(pk, p, nb, s1, dw, 0, st);
-                    else launch_pass<T, FFT_INV>(pk, p, nb, s2, dw, 0, st);
-                }
-                prof_set_category(QI_CAT_INV_LAST);
-                dim3 grid((unsigned)((N + CWTF_SPAN * CWTF_TILE - 1) / (CWTF_SPAN * CWTF_TILE)), (unsigned)gs, (unsigned)C);
-                QI_LAUNCH((cwtf_interp_kernel<T>), grid, dim3(256), 0, st, (const cplx<T>*)work, (const int*)(d_dec + sub),
-                          (const long long*)&d_bands[0].kc, (int)(sizeof(DevBand) / sizeof(long long)), geo, logD, cf,
-                          static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum);
-                sub += (size_t)gs;
-            }
-            pos = end;
-        }
-    }
+    int* d_dec = reinterpret_cast<int*>(base + lo.off_ids) + B;
+    T* coef = reinterpret_cast<T*>(base + lo.off_coef);
+    const auto dec_src = [&](const int* ids, int lk) { return SrcCwtDec<T>{spec, d_bands, ids, (int)C, lo.logL, lk, half_shift}; };
+    const int rc = decimated_route<T, true, true, 2>(fp.logK, geo, dec_src, &d_bands[0].kc, (int)(sizeof(DevBand) / sizeof(long long)),
+                                                     d_dec, coef, work, work, (size_t)lo.group * C * lo.L, out_c, out_p, band_sum, st);
+    if (rc != QI_OK) return rc;
 
     // ---- plain route: maximal runs of consecutive bands that took no other route
     for (int band0 = 0; band0 < B;) {
         if (fp.route[band0] != CWT_ROUTE_PLAIN) { ++band0; continue; }
         int g = 1;
         while (band0 + g < B && g < lo.group && fp.route[band0 + g] == CWT_ROUTE_PLAIN) ++g;
-        const i64 nb = (i64)g * C;
-        for (int p = np - 1; p >= 0; --p) {
-            const bool first = (p == np - 1), last = (p == 0);
-            SrcCwtSpec<T> s1{spec, tables, d_bands, band0, geo};
-            SrcComplex<T> s2{work, lo.L};
-            DstComplex<T> d1{work, lo.L, one};
-            DstCwtOut<T> d2{static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum, band0, geo, 0.0};
-            prof_set_category(last ? QI_CAT_INV_LAST : (first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID));
-            if (first && last) launch_pass<T, FFT_INV>(plan, p, nb, s1, d2, 256, st);
-            else if (first) launch_pass<T, FFT_INV>(plan, p, nb, s1, d1, 0, st);
-            else if (last) launch_pass<T, FFT_INV>(plan, p, nb, s2, d2, 256, st);
-            else launch_pass<T, FFT_INV>(plan, p, nb, s2, d1, 0, st);
-        }
+        inverse_passes<T>(plan, (i64)g * C, SrcCwtSpec<T>{spec, tables, d_bands, band0, geo},
+                          DstCwtOut<T>{static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum, band0, geo, 0.0}, 256,
+                          true, work, lo.L, st);
         band0 += g;
     }
     prof_set_category(QI_CAT_OTHER);

@@ -51,64 +51,26 @@ __global__ void cwtf_os_table_kernel(const DevBand* __restrict__ bandsF, int log
     tabF[((size_t)blockIdx.y << logF) + e] = gabor_response<T>(bandsF[blockIdx.y], k, logF, half_shift);
 }
 
-// grid: (ceil(N / V), channels); one block of F samples, all n_os bands.  dyn smem: (2 pad8(F) + F) complex + 256 B
-template <typename T>
-__global__ void __launch_bounds__(512)
-cwtf_os_kernel(const T* __restrict__ sig, i64 stride, CwtGeom geo, const int* __restrict__ ids, int n_os, int logF,
-               int half, const cplx<T>* __restrict__ tabF, cplx<T>* __restrict__ out_c, T* __restrict__ out_p,
-               double* __restrict__ band_sum) {
-    QI_DYN_SMEM(smem_raw);
-    const int F = 1 << logF, V = F - 2 * half;
-    const int FP = pad8(F);                                   // tiles in the padded single-column layout of tile_fft<.., true>
-    cplx<T>* tile_x = reinterpret_cast<cplx<T>*>(smem_raw);
-    cplx<T>* tile_y = tile_x + FP;
-    cplx<T>* tw = tile_y + FP;
-    double* scratch = reinterpret_cast<double*>(tw + F);
-    const i64 chan = blockIdx.y, N = geo.n_points;
-    const i64 n0 = (i64)blockIdx.x * V;
-    const T* xs = sig + chan * stride;
-    fill_stage_twiddles<T>(tw, logF);
-    for (int p = threadIdx.x; p < F; p += blockDim.x) {
-        const i64 k = n0 - half + p;
-        tile_x[padt<T>(p)] = mk<T>((k >= 0 && k < N) ? xs[k] : (T)0, (T)0);
-    }
-    __syncthreads();
-    tile_fft<T, FFT_FWD, true>(tile_x, tw, logF, 1, 1);
-    for (int i = 0; i < n_os; ++i) {
-        const int band = ids[i];
-        const cplx<T>* H = tabF + ((size_t)i << logF);
-        for (int r = threadIdx.x; r < F; r += blockDim.x) tile_y[padt<T>(r)] = tile_x[padt<T>(r)] * H[r];
-        __syncthreads();
-        tile_fft<T, FFT_INV, true>(tile_y, tw, logF, 1, 1);
-        const i64 row = (chan * geo.n_bands + band) * N;
-        double acc = 0.0;
-        for (int v = threadIdx.x; v < V; v += blockDim.x) {
-            const i64 n = n0 + v;
-            if (n < N) {
-                const cplx<T> y = tile_y[padt<T>(half + v)];
-                const T pw = norm2(y);
-                if (out_c) out_c[row + n] = y;
-                if (out_p) out_p[row + n] = pw;
-                acc += (double)pw;
-            }
-        }
-        if (band_sum) {
-            acc = block_sum(acc, scratch);
-            if (threadIdx.x == 0) atomicAdd(&band_sum[chan * geo.n_bands + band], acc);
-        }
-        __syncthreads();
-    }
-}
+// Gabor bands on the overlap-save route: the record zero-extended, the response from the bands' F-grid tables, the output
+// as the inverse transform leaves it
+template <typename T> struct OsTableRoute {
+    const cplx<T>* tabF;
+    struct Band {
+        const cplx<T>* H;
+        QI_DEV cplx<T> weigh(cplx<T> x, int r, const CwtGeom&) const { return x * H[r]; }
+        QI_DEV cplx<T> out(cplx<T> y, i64, const CwtGeom&) const { return y; }
+    };
+    QI_DEV T sample(const T* xs, i64 k, i64 N) const { return (k >= 0 && k < N) ? xs[k] : (T)0; }
+    QI_DEV Band band(int i, int) const { return Band{tabF + ((size_t)i << CWTF_OS_LOGF)}; }
+};
 
 // ---------------------------------------------------------------- host side: which band takes which route
 enum { CWT_ROUTE_PLAIN = 0, CWT_ROUTE_DEC = 1, CWT_ROUTE_OS = 2 };
 
 struct CwtFastPlan {
-    std::vector<int> route, logK;          // per band
-    std::vector<int> dec_ids;              // decimated bands ordered by logK
+    std::vector<int> route, logK;          // per band; logK < logL on the decimated route
     std::vector<int> os_ids;
     int os_half;
-    int n_plain;
 };
 
 template <typename T>
@@ -116,9 +78,8 @@ static void cwt_fast_plan(const QiAtomBand* hb, int B, i64 N, int logL, int conv
     typedef CwtFastCfg<T> Cfg;
     fp.route.assign(B, CWT_ROUTE_PLAIN);
     fp.logK.assign(B, logL);
-    fp.dec_ids.clear(); fp.os_ids.clear();
+    fp.os_ids.clear();
     fp.os_half = 0;
-    fp.n_plain = B;
     if (!enable || conv_mode != QI_CONV_LINEAR_SAME || logL < 14 || N < 4 * CWTF_TILE) return;
     const double L = (double)(1ll << logL);
     for (int b = 0; b < B; ++b) {
@@ -132,17 +93,10 @@ static void cwt_fast_plan(const QiAtomBand* hb, int B, i64 N, int logL, int conv
             if (half > fp.os_half) fp.os_half = half;
             continue;
         }
-        const double kmax = ceil(Cfg::U_CUT * L / (2.0 * M_PI * s)) + 1.0;
-        const double need = Cfg::RHO * (2.0 * kmax + 4.0);
-        int lk = logL - CWTF_MAX_LOGD;
-        if (lk < 6) lk = 6;
-        while (lk < logL && (double)(1ll << lk) < need) ++lk;
-        if (lk <= logL - 2) { fp.route[b] = CWT_ROUTE_DEC; fp.logK[b] = lk; }
+        fp.logK[b] = dec_logk(ceil(Cfg::U_CUT * L / (2.0 * M_PI * s)) + 1.0, Cfg::RHO, 4.0, logL, false);
+        if (fp.logK[b] < logL) fp.route[b] = CWT_ROUTE_DEC;
     }
-    for (int lk = 0; lk <= logL; ++lk)
-        for (int b = 0; b < B; ++b) if (fp.route[b] == CWT_ROUTE_DEC && fp.logK[b] == lk) fp.dec_ids.push_back(b);
     fp.os_half = (fp.os_half + 15) & ~15;
-    fp.n_plain = B - (int)fp.dec_ids.size() - (int)fp.os_ids.size();
 }
 
 }  // namespace qi

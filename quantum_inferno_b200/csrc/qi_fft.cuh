@@ -491,4 +491,32 @@ template <typename T> struct SrcRealPad {
     }
 };
 
+// ---------------------------------------------------------------- whole transforms
+// Forward transform of `nbatch` rows into `buf` (row stride `stride`, bit-reversed order): pass 0 reads `src`, the later
+// passes run on `buf` in place.
+template <typename T, class Src>
+inline void forward_passes(const FftPlan& plan, i64 nbatch, Src src, cplx<T>* buf, i64 stride, cudaStream_t st) {
+    const DstComplex<T> d{buf, stride, (T)1};
+    launch_pass<T, FFT_FWD>(plan, 0, nbatch, src, d, 0, st);
+    for (int p = 1; p < plan.npass; ++p) launch_pass<T, FFT_FWD>(plan, p, nbatch, SrcComplex<T>{buf, stride}, d, 0, st);
+}
+
+// Inverse transform of `nbatch` rows: the first pass (npass - 1) reads `src`, the last (0) writes `dst` with
+// `dst_scratch` bytes of sink scratch, and the passes between run on `buf` (row stride `stride`) in place.  The last pass
+// is timed as QI_CAT_INV_LAST when its sink writes the output planes (`dst_is_output`).
+template <typename T, class Src, class Dst>
+inline void inverse_passes(const FftPlan& plan, i64 nbatch, Src src, Dst dst, size_t dst_scratch, bool dst_is_output,
+                           cplx<T>* buf, i64 stride, cudaStream_t st) {
+    const SrcComplex<T> s_mid{buf, stride};
+    const DstComplex<T> d_mid{buf, stride, (T)1};
+    for (int p = plan.npass - 1; p >= 0; --p) {
+        const bool first = (p == plan.npass - 1), last = (p == 0);
+        prof_set_category(last && dst_is_output ? QI_CAT_INV_LAST : (first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID));
+        if (first && last) launch_pass<T, FFT_INV>(plan, p, nbatch, src, dst, dst_scratch, st);
+        else if (first) launch_pass<T, FFT_INV>(plan, p, nbatch, src, d_mid, 0, st);
+        else if (last) launch_pass<T, FFT_INV>(plan, p, nbatch, s_mid, dst, dst_scratch, st);
+        else launch_pass<T, FFT_INV>(plan, p, nbatch, s_mid, d_mid, 0, st);
+    }
+}
+
 }  // namespace qi

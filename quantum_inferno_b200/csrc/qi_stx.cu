@@ -34,8 +34,7 @@ template <typename T> struct SrcStxSpec {
     }
 };
 
-// Band-limited route (both dtypes; the float32-only method="multirate" further down predates it and keeps its packed
-// interpolator).  A Stockwell voice is a BASEBAND signal: X[k + shift] exp(-0.5 (q k)^2) is below exp(-0.5 U^2) of its peak
+// Band-limited route (both dtypes, and every decimated band of method="multirate").  A Stockwell voice is a BASEBAND signal: X[k + shift] exp(-0.5 (q k)^2) is below exp(-0.5 U^2) of its peak
 // beyond |k| > kmax = U / q.  The K = 2^m >= RHO (2 kmax + 4) bins around zero, inverse-transformed at length K, are the
 // voice at every D = n / K-th sample exactly; qi_interp.cuh brings it to the full rate (no carrier to put back).
 template <typename T> struct SrcStxDecT {
@@ -73,66 +72,30 @@ __global__ void stx_windows_kernel(const DevStxBand* bands, i64 n, cplx<T>* out)
 // record's) + one inverse transform in shared memory, the carrier taken out on the way to HBM.  Replaces two full-length
 // HBM passes per voice (a third of a Stockwell call at 16 x 2^18).  Truncating h at U_CUT sigma costs exp(-U_CUT^2 / 2)
 // (1.5e-7 float32, 1.3e-13 float64) of the peak, like the band-limited route.
-template <typename T>
-__global__ void __launch_bounds__(512)
-stx_os_kernel(const T* __restrict__ sig, i64 stride, CwtGeom geo, const DevStxBand* __restrict__ bands,
-              const int* __restrict__ ids, int n_os, int half, cplx<T>* __restrict__ out_c, T* __restrict__ out_p,
-              double* __restrict__ band_sum) {
-    QI_DYN_SMEM(smem_raw);
-    constexpr int logF = CWTF_OS_LOGF, F = 1 << logF;
-    const int V = F - 2 * half;
-    const int FP = pad8(F);
-    cplx<T>* tile_x = reinterpret_cast<cplx<T>*>(smem_raw);
-    cplx<T>* tile_y = tile_x + FP;
-    cplx<T>* tw = tile_y + FP;
-    double* scratch = reinterpret_cast<double*>(tw + F);
-    const i64 chan = blockIdx.y, N = geo.n_points;                  // N = 2^logL
-    const i64 n0 = (i64)blockIdx.x * V;
-    const T* xs = sig + chan * stride;
-    fill_stage_twiddles<T>(tw, logF);
-    for (int p = threadIdx.x; p < F; p += blockDim.x)
-        tile_x[padt<T>(p)] = mk<T>(xs[(n0 - half + p) & (N - 1)], (T)0);       // circular, like the reference's product
-    __syncthreads();
-    tile_fft<T, FFT_FWD, true>(tile_x, tw, logF, 1, 1);
-    const int up = geo.logL - logF;                                   // block bin j <-> record bin j << up
-    for (int i = 0; i < n_os; ++i) {
-        const int band = ids[i];
-        const DevStxBand b = bands[band];
-        for (int r = threadIdx.x; r < F; r += blockDim.x) {
-            const i64 j = (i64)brev_bits((unsigned)r, logF);
-            i64 u = ((j << up) - b.shift) & (N - 1);
-            if (u >= (N >> 1)) u -= N;                                // signed distance from the voice's centre bin
+template <typename T> struct OsStxRoute {
+    const DevStxBand* bands;
+    struct Band {
+        DevStxBand b;
+        QI_DEV cplx<T> weigh(cplx<T> x, int r, const CwtGeom& geo) const {
+            const i64 N = geo.n_points;                                  // 2^logL
+            const i64 j = (i64)brev_bits((unsigned)r, CWTF_OS_LOGF);    // block bin j <-> record bin j << (logL - logF)
+            i64 u = ((j << (geo.logL - CWTF_OS_LOGF)) - b.shift) & (N - 1);
+            if (u >= (N >> 1)) u -= N;                                  // signed distance from the voice's centre bin
             T w = (T)0;
             if (u <= b.kmax && -u <= b.kmax) {
                 const T a = (T)b.q * (T)u;
-                w = exp((T)-0.5 * a * a) * (T)(1.0 / (double)F);
+                w = exp((T)-0.5 * a * a) * (T)(1.0 / (double)(1 << CWTF_OS_LOGF));
             }
-            tile_y[padt<T>(r)] = tile_x[padt<T>(r)] * w;
+            return x * w;
         }
-        __syncthreads();
-        tile_fft<T, FFT_INV, true>(tile_y, tw, logF, 1, 1);
-        const i64 row = (chan * geo.n_bands + band) * N;
-        double acc = 0.0;
-        for (int v = threadIdx.x; v < V; v += blockDim.x) {
-            const i64 n = n0 + v;
-            if (n < N) {
-                const cplx<T> y = tile_y[padt<T>(half + v)];
-                const T pw = norm2(y);
-                if (out_c) {
-                    const unsigned long long m = ((unsigned long long)b.shift * (unsigned long long)n) & (unsigned long long)(N - 1);
-                    out_c[row + n] = mul_conj(y, unit_root<T>(m, geo.logL));       // * exp(-2 pi i shift n / N), exact phase
-                }
-                if (out_p) out_p[row + n] = pw;
-                acc += (double)pw;
-            }
+        QI_DEV cplx<T> out(cplx<T> y, i64 n, const CwtGeom& geo) const {   // * exp(-2 pi i shift n / N), exact phase
+            const unsigned long long m = ((unsigned long long)b.shift * (unsigned long long)n) & (unsigned long long)(geo.n_points - 1);
+            return mul_conj(y, unit_root<T>(m, geo.logL));
         }
-        if (band_sum) {
-            acc = block_sum(acc, scratch);
-            if (threadIdx.x == 0) atomicAdd(&band_sum[chan * geo.n_bands + band], acc);
-        }
-        __syncthreads();
-    }
-}
+    };
+    QI_DEV T sample(const T* xs, i64 k, i64 N) const { return xs[k & (N - 1)]; }   // circular, like the reference's product
+    QI_DEV Band band(int, int band) const { return Band{bands[band]}; }
+};
 
 struct StxLayout { int logL; i64 L; size_t off_bands, off_spec, off_work, off_ids, off_coef, total; int group; };
 
@@ -171,6 +134,30 @@ static void upload_stx_bands(const QiStxBand* hb, int B, i64 N, double u_zero, D
     stage_to_device(d_bands, db.data(), sizeof(DevStxBand) * (size_t)B, st);
 }
 
+static CwtGeom stx_geom(i64 C, i64 N, int B, int logL) {
+    CwtGeom geo;
+    geo.n_points = N; geo.n_channels = C; geo.n_bands = B; geo.logL = logL;
+    geo.conv_mode = QI_CONV_LINEAR_SAME; geo.fs = 0; geo.centre_idx = 0; geo.half_shift = 0; geo.d_min = 0; geo.d_max = 0;
+    return geo;
+}
+
+// full-length passes over maximal runs of at most `group` consecutive bands b with logK[b] == logL
+template <typename T>
+static void stx_full_length(const FftPlan& plan, const std::vector<int>& logK, int group, const cplx<T>* spec,
+                            const DevStxBand* d_bands, cplx<T>* work, const CwtGeom& geo, void* out_c, void* out_p,
+                            double* band_sum, cudaStream_t st) {
+    const int B = (int)logK.size();
+    for (int band0 = 0; band0 < B;) {
+        if (logK[band0] != geo.logL) { ++band0; continue; }
+        int g = 1;
+        while (band0 + g < B && g < group && logK[band0 + g] == geo.logL) ++g;
+        inverse_passes<T>(plan, (i64)g * geo.n_channels, SrcStxSpec<T>{spec, d_bands, band0, geo},
+                          DstCwtOut<T>{static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum, band0, geo, 0.0}, 256,
+                          true, work, geo.n_points, st);
+        band0 += g;
+    }
+}
+
 template <typename T>
 static int stx_fft_impl(const void* sig, i64 C, i64 N, i64 stride, const QiStxBand* hb, int B, void* out_c,
                         void* out_p, double* band_sum, void* ws, size_t ws_bytes, int group, cudaStream_t st, bool fast) {
@@ -182,85 +169,29 @@ static int stx_fft_impl(const void* sig, i64 C, i64 N, i64 stride, const QiStxBa
     DevStxBand* d_bands = reinterpret_cast<DevStxBand*>(base + lo.off_bands);
     cplx<T>* spec = reinterpret_cast<cplx<T>*>(base + lo.off_spec);
     cplx<T>* work = reinterpret_cast<cplx<T>*>(base + lo.off_work);
+    int* d_ids = reinterpret_cast<int*>(base + lo.off_ids);
     upload_stx_bands(hb, B, N, sizeof(T) == 4 ? 14.5 : 38.7, d_bands, st, Cfg::U_CUT);
-
-    CwtGeom geo;
-    geo.n_points = N; geo.n_channels = C; geo.n_bands = B; geo.logL = lo.logL;
-    geo.conv_mode = QI_CONV_LINEAR_SAME; geo.fs = 0; geo.centre_idx = 0; geo.half_shift = 0; geo.d_min = 0; geo.d_max = 0;
-
+    const CwtGeom geo = stx_geom(C, N, B, lo.logL);
     const FftPlan plan = make_plan(lo.logL, (int)sizeof(cplx<T>));
-    const int np = plan.npass;
-    const T one = (T)1;
     prof_set_category(QI_CAT_FFT_FWD);
-    for (int p = 0; p < np; ++p) {
-        DstComplex<T> d{spec, lo.L, one};
-        if (p == 0) {
-            SrcRealPad<T> s{static_cast<const T*>(sig), stride, N};
-            launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st);
-        } else {
-            SrcComplex<T> s{spec, lo.L};
-            launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st);
-        }
-    }
+    forward_passes<T>(plan, C, SrcRealPad<T>{static_cast<const T*>(sig), stride, N}, spec, lo.L, st);
     if (band_sum) cudaMemsetAsync(band_sum, 0, sizeof(double) * (size_t)C * B, st);
     // ---- band-limited route: bands whose window fits K <= n / 4 bins, grouped by K
-    std::vector<int> logK(B, lo.logL), dec_ids;
+    std::vector<int> logK(B, lo.logL);
+    int n_dec = 0;
     if (fast && lo.logL >= 13) {
         for (int b = 0; b < B; ++b) {
             const double aq = fabs(hb[b].sigma * 2.0 * M_PI / (double)N);
             if (!(aq > 0.0)) continue;
-            const double need = Cfg::RHO * (2.0 * (ceil(Cfg::U_CUT / aq) + 1.0) + 4.0);
-            int lk = lo.logL - CWTF_MAX_LOGD;
-            if (lk < 6) lk = 6;
-            while (lk < lo.logL && (double)(1ll << lk) < need) ++lk;
-            if (lk <= lo.logL - 2) logK[b] = lk;
-        }
-        for (int lk = 0; lk < lo.logL; ++lk)
-            for (int b = 0; b < B; ++b) if (logK[b] == lk) dec_ids.push_back(b);
-    }
-    if (!dec_ids.empty()) {
-        int* d_ids = reinterpret_cast<int*>(base + lo.off_ids);
-        T* coef = reinterpret_cast<T*>(base + lo.off_coef);
-        stage_to_device(d_ids, dec_ids.data(), sizeof(int) * dec_ids.size(), st);
-        unsigned need_mask = 0;
-        for (int b : dec_ids) need_mask |= 1u << (lo.logL - logK[b]);
-        prof_set_category(QI_CAT_OTHER);
-        QI_LAUNCH((cwtf_coef_kernel<T>), dim3((unsigned)((Cfg::TAPS << CWTF_MAX_LOGD) / 256 + 1), (unsigned)(CWTF_MAX_LOGD + 1)),
-                  dim3(256), 0, st, coef, need_mask, 1.0 / cwtf_bessel_i0(Cfg::BETA));
-        const size_t work_elems = (size_t)lo.group * C * lo.L;
-        size_t pos = 0;
-        while (pos < dec_ids.size()) {
-            const int lk = logK[dec_ids[pos]];
-            size_t end = pos;
-            while (end < dec_ids.size() && logK[dec_ids[end]] == lk) ++end;
-            const int logD = lo.logL - lk;
-            const T* cf = coef + (size_t)logD * Cfg::TAPS * (1u << CWTF_MAX_LOGD);
-            const FftPlan pk = make_plan(lk, (int)sizeof(cplx<T>));
-            const i64 K = 1ll << lk;
-            for (size_t sub = pos; sub < end;) {
-                i64 gs = (i64)(end - sub);
-                while (gs > 1 && (gs * C > 65535 || (size_t)gs * C * K > work_elems)) --gs;
-                if (gs * C > 65535 || (size_t)gs * C * K > work_elems) return QI_ERR_WORKSPACE;
-                const i64 nbd = gs * C;
-                SrcStxDecT<T> s1{spec, d_bands, d_ids + sub, (int)C, lo.logL, lk};
-                for (int p = pk.npass - 1; p >= 0; --p) {
-                    const bool first = (p == pk.npass - 1);
-                    SrcComplex<T> s2{work, K};
-                    DstComplex<T> dw{work, K, one};
-                    prof_set_category(first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID);
-                    if (first) launch_pass<T, FFT_INV>(pk, p, nbd, s1, dw, 0, st);
-                    else launch_pass<T, FFT_INV>(pk, p, nbd, s2, dw, 0, st);
-                }
-                prof_set_category(QI_CAT_INV_LAST);
-                dim3 grid((unsigned)((N + CWTF_SPAN * CWTF_TILE - 1) / (CWTF_SPAN * CWTF_TILE)), (unsigned)gs, (unsigned)C);
-                QI_LAUNCH((cwtf_interp_kernel<T>), grid, dim3(256), 0, st, (const cplx<T>*)work, (const int*)(d_ids + sub),
-                          (const long long*)nullptr, 0, geo, logD, cf, static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p),
-                          band_sum);
-                sub += (size_t)gs;
-            }
-            pos = end;
+            logK[b] = dec_logk(ceil(Cfg::U_CUT / aq) + 1.0, Cfg::RHO, 4.0, lo.logL, false);
+            if (logK[b] < lo.logL) ++n_dec;
         }
     }
+    T* coef = reinterpret_cast<T*>(base + lo.off_coef);
+    const auto dec_src = [&](const int* ids, int lk) { return SrcStxDecT<T>{spec, d_bands, ids, (int)C, lo.logL, lk}; };
+    const int rc = decimated_route<T, false, true, 2>(logK, geo, dec_src, nullptr, 0, d_ids, coef, work, work,
+                                                      (size_t)lo.group * C * lo.L, out_c, out_p, band_sum, st);
+    if (rc != QI_OK) return rc;
     // ---- overlap-save route: voices that are too wide to decimate and short in time
     if (fast && lo.logL >= 13) {
         std::vector<int> os_ids;
@@ -274,386 +205,146 @@ static int stx_fft_impl(const void* sig, i64 C, i64 N, i64 stride, const QiStxBa
             if (sg >= 2.5 && half <= CWTF_OS_MAX_HALF) { os_ids.push_back(b); if (half > os_half) os_half = half; }
         }
         if (!os_ids.empty()) {
-            os_half = (os_half + 15) & ~15;
-            int* d_os = reinterpret_cast<int*>(base + lo.off_ids) + dec_ids.size();
+            int* d_os = d_ids + n_dec;
             stage_to_device(d_os, os_ids.data(), sizeof(int) * os_ids.size(), st);
-            for (int b : os_ids) logK[b] = -1;                          // taken: the full-length loop below skips them
-            const int F = 1 << CWTF_OS_LOGF, V = F - 2 * os_half;
-            const size_t smem = sizeof(cplx<T>) * (2 * (size_t)pad8(F) + (size_t)F) + 256;
-#ifndef QI_EMUL
-            cudaFuncSetAttribute(stx_os_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-#endif
-            prof_set_category(QI_CAT_INV_LAST);
-            QI_LAUNCH((stx_os_kernel<T>), dim3((unsigned)((N + V - 1) / V), (unsigned)C), dim3(512), smem, st,
-                      static_cast<const T*>(sig), stride, geo, (const DevStxBand*)d_bands, (const int*)d_os, (int)os_ids.size(),
-                      os_half, static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum);
+            for (int b : os_ids) logK[b] = -1;                          // taken: the full-length passes skip them
+            overlap_save_route<T>(sig, stride, geo, d_os, (int)os_ids.size(), (os_half + 15) & ~15, OsStxRoute<T>{d_bands},
+                                  out_c, out_p, band_sum, st);
         }
     }
-    // ---- full-length passes: maximal runs of consecutive bands that took no other route
-    for (int band0 = 0; band0 < B;) {
-        if (logK[band0] != lo.logL) { ++band0; continue; }
-        int g = 1;
-        while (band0 + g < B && g < lo.group && logK[band0 + g] == lo.logL) ++g;
-        const i64 nb = (i64)g * C;
-        for (int p = np - 1; p >= 0; --p) {
-            const bool first = (p == np - 1), last = (p == 0);
-            SrcStxSpec<T> s1{spec, d_bands, band0, geo};
-            SrcComplex<T> s2{work, lo.L};
-            DstComplex<T> d1{work, lo.L, one};
-            DstCwtOut<T> d2{static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), band_sum, band0, geo, 0.0};
-            prof_set_category(last ? QI_CAT_INV_LAST : (first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID));
-            if (first && last) launch_pass<T, FFT_INV>(plan, p, nb, s1, d2, 256, st);
-            else if (first) launch_pass<T, FFT_INV>(plan, p, nb, s1, d1, 0, st);
-            else if (last) launch_pass<T, FFT_INV>(plan, p, nb, s2, d2, 256, st);
-            else launch_pass<T, FFT_INV>(plan, p, nb, s2, d1, 0, st);
-        }
-        band0 += g;
-    }
+    // ---- full-length passes: the bands that took no other route
+    stx_full_length<T>(plan, logK, lo.group, spec, d_bands, work, geo, out_c, out_p, band_sum, st);
     prof_set_category(QI_CAT_OTHER);
     return check_cuda("qi_stx_fft");
 }
 
 
 // ---------------------------------------------------------------- multirate (float32) Stockwell
-// A Stockwell voice is a BASEBAND signal: its spectrum X[k + shift] * exp(-0.5 (q k)^2) is below 2.7e-7 of its peak
-// beyond |k| > kmax = 5.5 / q.  The K = 2^m >= 4 kmax bins around zero therefore give, by an inverse transform of
-// length K, the samples of the voice at every D = n / K-th output exactly (2x oversampled), and a 16-tap-per-phase
-// Kaiser-windowed-sinc interpolator (beta = 11.2, stop band -110 dB) brings them to the full rate:
-//     out[m D + p] = sum_{j=0..15} h(p - (j - 7) D) * dec[(m - 7 + j) mod K],   h(t) = sinc(t / D) * kaiser(t / 8D)
-// (circular, like the reference's product).  Traffic: 8 B per cell written + 16 / D read, instead of two full-length
-// passes of 16 B each way.  Bands too wide to decimate (K = n) keep the exact passes.  numpy model and error budget:
+// The exact path's pieces under another plan: every band whose voice fits K <= n / 2 bins at a 5.5-sigma cut (2.7e-7 of
+// its peak; K = 2^m >= 4 kmax + 4, i.e. the decimated samples 2x oversampled) takes the decimated route, the rest the
+// full-length passes; no overlap-save route and no band sums.  numpy model and error budget:
 // tools/stx_multirate_prototype.py; measured against the full-length transform: relative L2 3e-6, max 6e-6.
-constexpr int STXMR_TAPS = 16;
-constexpr int STXMR_MAX_LOGD = 8;
-constexpr int STXMR_TILE = 2048;
-constexpr int STXMR_SPAN = 4;                 // tiles per CTA of the interpolator (coefficients loaded once)
 constexpr double STXMR_U = 5.5;
-constexpr double STXMR_BETA = 11.2;
 
-struct SrcStxDec {
-    const cplx<float>* spec; const DevStxBand* bands; const int* ids; int n_channels, logN, logK;
-    QI_DEV cplx<float> load(i64 batch, i64 e) const {
-        const i64 chan = batch % n_channels;
-        const DevStxBand b = bands[ids[batch / n_channels]];
-        const i64 K = 1ll << logK, n = 1ll << logN;
-        const i64 k = (i64)brev_bits((unsigned)e, logK);
-        const i64 ks = (k < (K >> 1)) ? k : k - K;
-        if (ks > b.kmax || -ks > b.kmax) return mk<float>(0.0f, 0.0f);
-        const i64 ksrc = (ks + b.shift) & (n - 1);
-        const cplx<float> X = spec[(chan << logN) + (i64)brev_bits((unsigned)ksrc, logN)];
-        const float u = (float)b.q * (float)ks;
-        return X * (expf(-0.5f * u * u) * (float)(1.0 / (double)n));
+struct StxMrLayout { size_t off_bands, off_ids, off_spec, off_work, off_dec, off_coef, total, dec_elems; i64 gx; };
+
+static StxMrLayout stxmr_layout(i64 C, i64 N, const QiStxBand* hb, int B, std::vector<int>& logK) {
+    StxMrLayout lo;
+    const int logN = ceil_log2_i64(N);
+    size_t dec_elems = 0;
+    int count[64] = {0};
+    logK.resize(B);
+    for (int b = 0; b < B; ++b) {
+        logK[b] = dec_logk(ceil(STXMR_U / fabs(hb[b].sigma * 2.0 * M_PI / (double)N)) + 1.0, 2.0, 2.0, logN, true);
+        ++count[logK[b]];
     }
-};
-
-// modified Bessel function I0 by its power series (32 terms: below 1e-19 of the sum for x <= 11.2)
-QI_HD double stxmr_bessel_i0(double x) {
-    double s = 1.0, term = 1.0;
-    const double hh = 0.25 * x * x;
-    for (int k = 1; k <= 32; ++k) { term *= hh / (double)(k * k); s += term; }
-    return s;
+    for (int lk = 0; lk < logN; ++lk) {
+        const size_t e = (size_t)count[lk] * (size_t)C << lk;
+        dec_elems = e > dec_elems ? e : dec_elems;
+    }
+    i64 gx = (i64)((1ull << 30) / ((size_t)C * (size_t)N * sizeof(cplx<float>)));   // exact bands per launch: <= 1 GiB of scratch
+    if (gx < 1) gx = 1;
+    if (gx > count[logN]) gx = count[logN] > 0 ? count[logN] : 1;
+    while (gx * C > 65535 && gx > 1) --gx;
+    lo.gx = gx;
+    lo.dec_elems = dec_elems;
+    const size_t work_elems = dec_elems > (size_t)gx * C * N ? dec_elems : (size_t)gx * C * N;
+    size_t o = 0;
+    lo.off_bands = o; o = align_up(o + sizeof(DevStxBand) * (size_t)B, 256);
+    lo.off_ids = o; o = align_up(o + sizeof(int) * (size_t)B, 256);
+    lo.off_spec = o; o = align_up(o + sizeof(cplx<float>) * (size_t)C * N, 256);
+    lo.off_work = o; o = align_up(o + sizeof(cplx<float>) * work_elems, 256);
+    lo.off_dec = o; o = align_up(o + sizeof(cplx<float>) * (dec_elems ? dec_elems : 1), 256);
+    lo.off_coef = o; o = align_up(o + sizeof(float) * CwtFastCfg<float>::TAPS * (size_t)(CWTF_MAX_LOGD + 1) * (1u << CWTF_MAX_LOGD), 256);
+    lo.total = o;
+    return lo;
 }
 
-// table of decimation 2^logD (logD = blockIdx.y, slot logD of `coef_all`): coef[j * D + p] = h(p - (j - 7) D)
-__global__ void stxmr_coef_kernel(float* __restrict__ coef_all, unsigned need_mask, double inv_i0_beta) {
-    const int logD = blockIdx.y;
-    if (!((need_mask >> logD) & 1u)) return;
-    float* coef = coef_all + (size_t)logD * STXMR_TAPS * (1u << STXMR_MAX_LOGD);
-    const int D = 1 << logD;
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= STXMR_TAPS * D) return;
-    const int j = idx >> logD, p = idx & (D - 1);
-    const double t = (double)(p - (j - 7) * D);
-    const double x = t / (8.0 * D);
-    const double arg = 1.0 - x * x;
-    const double w = stxmr_bessel_i0(STXMR_BETA * sqrt(arg > 0.0 ? arg : 0.0)) * inv_i0_beta;
-    const double y = t / (double)D;
-    const double sinc = t == 0.0 ? 1.0 : sinpi(y) / (M_PI * y);
-    coef[idx] = (float)(sinc * w);
+static int stx_multirate_impl(const void* sig, i64 C, i64 N, i64 stride, const QiStxBand* hb, int B, void* out_c, void* out_p,
+                              void* ws, size_t ws_bytes, cudaStream_t st) {
+    typedef float T;
+    const int logN = ceil_log2_i64(N);
+    std::vector<int> logK;
+    const StxMrLayout lo = stxmr_layout(C, N, hb, B, logK);
+    if (ws_bytes < lo.total) return QI_ERR_WORKSPACE;
+    unsigned char* base = static_cast<unsigned char*>(ws);
+    DevStxBand* d_bands = reinterpret_cast<DevStxBand*>(base + lo.off_bands);
+    cplx<T>* spec = reinterpret_cast<cplx<T>*>(base + lo.off_spec);
+    cplx<T>* work = reinterpret_cast<cplx<T>*>(base + lo.off_work);
+    cplx<T>* dec = reinterpret_cast<cplx<T>*>(base + lo.off_dec);
+    int* d_ids = reinterpret_cast<int*>(base + lo.off_ids);
+    T* coef = reinterpret_cast<T*>(base + lo.off_coef);
+    // decimated bands are cut at 5.5 sigma (dec_kmax), the full-length ones at the float32 underflow point (kmax)
+    upload_stx_bands(hb, B, N, 14.5, d_bands, st, STXMR_U);
+    const CwtGeom geo = stx_geom(C, N, B, logN);
+    const FftPlan plan = make_plan(logN, (int)sizeof(cplx<T>));
+    prof_set_category(QI_CAT_FFT_FWD);
+    forward_passes<T>(plan, C, SrcRealPad<T>{static_cast<const T*>(sig), stride, N}, spec, N, st);
+    const auto dec_src = [&](const int* ids, int lk) { return SrcStxDecT<T>{spec, d_bands, ids, (int)C, logN, lk}; };
+    const int rc = decimated_route<T, false, false, 1>(logK, geo, dec_src, nullptr, 0, d_ids, coef, work, dec, lo.dec_elems,
+                                                       out_c, out_p, nullptr, st);
+    if (rc != QI_OK) return rc;
+    // bands too wide to decimate: runs of consecutive band indices, at most gx per launch
+    stx_full_length<T>(plan, logK, (int)lo.gx, spec, d_bands, work, geo, out_c, out_p, nullptr, st);
+    prof_set_category(QI_CAT_OTHER);
+    return check_cuda("qi_stx_multirate");
 }
 
-// grid: (ceil(n / (STXMR_SPAN * STXMR_TILE)), bands of the group, channels)
-__global__ void __launch_bounds__(256)
-stxmr_interp_kernel(const cplx<float>* __restrict__ dec, const int* __restrict__ ids, int n_channels, int n_bands, int logN,
-                    int logD, const float* __restrict__ coef, cplx<float>* __restrict__ out_c, float* __restrict__ out_p) {
-    // one pad slot per 8 decimated samples: at small D the lanes of a warp start their windows 8 samples apart
-    __shared__ cplx<float> seg[(STXMR_SPAN * STXMR_TILE / 2 + STXMR_TAPS) * 9 / 8 + 2];
-    const int D = 1 << logD, logK = logN - logD;
-    const i64 K = 1ll << logK, N = 1ll << logN;
-    const i64 span0 = (i64)blockIdx.x * (STXMR_SPAN * STXMR_TILE);
-    const i64 left = (N - span0) / STXMR_TILE;
-    const int ntile = left < STXMR_SPAN ? (int)left : STXMR_SPAN;
-    const int bi = blockIdx.y, chan = blockIdx.z, band = ids[bi];
-    const cplx<float>* src = dec + (((i64)bi * n_channels + chan) << logK);
-    const i64 m_base = (span0 >> logD) - 7;
-    const int nseg = ((ntile * STXMR_TILE) >> logD) + STXMR_TAPS;
-    for (int i = threadIdx.x; i < nseg; i += blockDim.x) seg[i + (i >> 3)] = src[(m_base + i) & (K - 1)];
-    __syncthreads();
-    const i64 row = ((i64)chan * n_bands + band) << logN;
-    // Thread (p, g): phase p = tid mod D, and the 8 consecutive decimated positions m = 8 g .. 8 g + 7 (256 / D threads
-    // share a phase).  Its sixteen coefficients and the 23 decimated samples under its window stay in registers: one
-    // shared-memory load per 1.4 outputs instead of 16 per output.
-    constexpr int PER = STXMR_TILE / 256;                             // outputs per thread
-    const int p = threadIdx.x & (D - 1), mg = (threadIdx.x >> logD) * PER;
-#ifndef QI_EMUL
-    // (re, im) pairs go through the packed fma.rn.f32x2 with the coefficient duplicated in both halves: 16 instead of 32
-    // FMA instructions per output
-    unsigned long long cf2[STXMR_TAPS], win2[PER + STXMR_TAPS - 1];
-#pragma unroll
-    for (int j = 0; j < STXMR_TAPS; ++j) {
-        const float c = coef[(j << logD) + p];
-        asm("mov.b64 %0, {%1, %2};" : "=l"(cf2[j]) : "f"(c), "f"(c));
-    }
-    for (int tl = 0; tl < ntile; ++tl) {
-        const int m0 = tl * (STXMR_TILE >> logD) + mg;
-        const i64 tile0 = span0;
-#pragma unroll
-        for (int j = 0; j < PER + STXMR_TAPS - 1; ++j) win2[j] = *reinterpret_cast<const unsigned long long*>(&seg[m0 + j + ((m0 + j) >> 3)]);
-#pragma unroll
-        for (int i = 0; i < PER; ++i) {
-            unsigned long long acc;
-            asm("mov.b64 %0, {%1, %1};" : "=l"(acc) : "f"(0.0f));
-#pragma unroll
-            for (int j = 0; j < STXMR_TAPS; ++j) asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(cf2[j]), "l"(win2[i + j]));
-            float re, im;
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(re), "=f"(im) : "l"(acc));
-            const i64 o = row + tile0 + ((i64)(m0 + i) << logD) + p;
-            if (out_c) out_c[o] = mk<float>(re, im);
-            if (out_p) out_p[o] = re * re + im * im;
-        }
-    }
-#else
-        float cf[STXMR_TAPS];
-#pragma unroll
-        for (int j = 0; j < STXMR_TAPS; ++j) cf[j] = coef[(j << logD) + p];
-    for (int tl = 0; tl < ntile; ++tl) {
-        const int m0 = tl * (STXMR_TILE >> logD) + mg;
-        const i64 tile0 = span0;
-        cplx<float> win[PER + STXMR_TAPS - 1];
-#pragma unroll
-        for (int j = 0; j < PER + STXMR_TAPS - 1; ++j) win[j] = seg[m0 + j + ((m0 + j) >> 3)];
-#pragma unroll
-        for (int i = 0; i < PER; ++i) {
-            float re = 0.0f, im = 0.0f;
-#pragma unroll
-            for (int j = 0; j < STXMR_TAPS; ++j) {
-                re += cf[j] * win[i + j].re;
-                im += cf[j] * win[i + j].im;
-            }
-            const i64 o = row + tile0 + ((i64)(m0 + i) << logD) + p;
-            if (out_c) out_c[o] = mk<float>(re, im);
-            if (out_p) out_p[o] = re * re + im * im;
-        }
-    }
-#endif
-        (void)N;
-    }
+template <typename T>
+static int stx_windows_impl(const QiStxBand* hb, int B, i64 N, void* out, void* ws, size_t ws_bytes, cudaStream_t st) {
+    if (ws_bytes < sizeof(DevStxBand) * (size_t)B) return QI_ERR_WORKSPACE;
+    DevStxBand* d_bands = static_cast<DevStxBand*>(ws);
+    upload_stx_bands(hb, B, N, 1e300, d_bands, st);
+    dim3 grid((unsigned)((N + 255) / 256), (unsigned)B);
+    QI_LAUNCH((stx_windows_kernel<T>), grid, dim3(256), 0, st, d_bands, N, static_cast<cplx<T>*>(out));
+    return check_cuda("qi_stx_windows");
+}
 
-    struct StxMrBandPlan { int logK; };
+}  // namespace qi
 
-    struct StxMrLayout { size_t off_bands, off_ids, off_spec, off_work, off_dec, off_coef, total; i64 gx; };
+extern "C" {
 
-    static int stxmr_logk(double q, i64 N, int logN) {
-        const double kmax = ceil(STXMR_U / fabs(q)) + 1.0;
-        int logK = logN - STXMR_MAX_LOGD;
-        if (logK < 6) logK = 6;
-        while (logK < logN && (double)(1ll << logK) < 4.0 * kmax + 4.0) ++logK;
-        return logK;
-    }
+size_t qi_stx_workspace_bytes(int64_t C, int64_t N, int B, int group, int dtype) {
+    if (C <= 0 || N <= 0 || B <= 0) return 0;
+    if (group < 0) group = -group;
+    return dtype == QI_F32 ? qi::stx_layout<float>(C, N, B, group).total : qi::stx_layout<double>(C, N, B, group).total;
+}
 
-    static StxMrLayout stxmr_layout(i64 C, i64 N, const QiStxBand* hb, int B) {
-        StxMrLayout lo;
-        const int logN = ceil_log2_i64(N);
-        size_t dec_elems = 0;
-        int count[64] = {0};
-        for (int b = 0; b < B; ++b) ++count[stxmr_logk(hb[b].sigma * 2.0 * M_PI / (double)N, N, logN)];
-        for (int lk = 0; lk < logN; ++lk) {
-            const size_t e = (size_t)count[lk] * (size_t)C << lk;
-            dec_elems = e > dec_elems ? e : dec_elems;
-        }
-        i64 gx = (i64)((1ull << 30) / ((size_t)C * (size_t)N * sizeof(cplx<float>)));   // exact bands per launch: <= 1 GiB of scratch
-        if (gx < 1) gx = 1;
-        if (gx > count[logN]) gx = count[logN] > 0 ? count[logN] : 1;
-        while (gx * C > 65535 && gx > 1) --gx;
-        lo.gx = gx;
-        const size_t work_elems = dec_elems > (size_t)gx * C * N ? dec_elems : (size_t)gx * C * N;
-        size_t o = 0;
-        lo.off_bands = o; o = align_up(o + sizeof(DevStxBand) * (size_t)B, 256);
-        lo.off_ids = o; o = align_up(o + sizeof(int) * (size_t)B, 256);
-        lo.off_spec = o; o = align_up(o + sizeof(cplx<float>) * (size_t)C * N, 256);
-        lo.off_work = o; o = align_up(o + sizeof(cplx<float>) * work_elems, 256);
-        lo.off_dec = o; o = align_up(o + sizeof(cplx<float>) * (dec_elems ? dec_elems : 1), 256);
-        lo.off_coef = o; o = align_up(o + sizeof(float) * STXMR_TAPS * (size_t)(STXMR_MAX_LOGD + 1) * (1u << STXMR_MAX_LOGD), 256);
-        lo.total = o;
-        return lo;
-    }
+int qi_stx_fft(const void* sig, int64_t C, int64_t N, int64_t stride, const QiStxBand* bands, int B, int dtype,
+               void* out_tfr, void* out_power, double* band_sum, void* ws, size_t ws_bytes, int group, void* stream) {
+    if (!sig || !bands || !ws || C <= 0 || N <= 0 || B <= 0 || stride < N) return QI_ERR_ARG;
+    if (N & (N - 1)) return QI_ERR_ARG;
+    if (N > (1ll << 30)) return QI_ERR_UNSUPPORTED;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const bool fast = group >= 0;                  // a negative bands_per_group keeps every band on the full-length passes
+    if (group < 0) group = -group;
+    if (dtype == QI_F32) return qi::stx_fft_impl<float>(sig, C, N, stride, bands, B, out_tfr, out_power, band_sum, ws, ws_bytes, group, st, fast);
+    if (dtype == QI_F64) return qi::stx_fft_impl<double>(sig, C, N, stride, bands, B, out_tfr, out_power, band_sum, ws, ws_bytes, group, st, fast);
+    return QI_ERR_ARG;
+}
 
-    static int stx_multirate_impl(const void* sig, i64 C, i64 N, i64 stride, const QiStxBand* hb, int B, void* out_c, void* out_p,
-                                  void* ws, size_t ws_bytes, cudaStream_t st) {
-        typedef float T;
-        const int logN = ceil_log2_i64(N);
-        const StxMrLayout lo = stxmr_layout(C, N, hb, B);
-        if (ws_bytes < lo.total) return QI_ERR_WORKSPACE;
-        unsigned char* base = static_cast<unsigned char*>(ws);
-        DevStxBand* d_bands = reinterpret_cast<DevStxBand*>(base + lo.off_bands);
-        int* d_ids = reinterpret_cast<int*>(base + lo.off_ids);
-        cplx<T>* spec = reinterpret_cast<cplx<T>*>(base + lo.off_spec);
-        cplx<T>* work = reinterpret_cast<cplx<T>*>(base + lo.off_work);
-        cplx<T>* dec = reinterpret_cast<cplx<T>*>(base + lo.off_dec);
-        float* coef = reinterpret_cast<float*>(base + lo.off_coef);
+size_t qi_stx_multirate_workspace_bytes(int64_t C, int64_t N, const QiStxBand* bands, int B) {
+    if (C <= 0 || N < 2 * qi::CWTF_TILE || (N & (N - 1)) || B <= 0 || !bands) return 0;
+    std::vector<int> logK;
+    return qi::stxmr_layout(C, N, bands, B, logK).total;
+}
 
-        // band table (decimated bands carry the 5.5-sigma cut-off, exact bands the float32 underflow point) and the band
-        // ids ordered by transform length
-        std::vector<DevStxBand> db(B);
-        std::vector<int> logk(B), ids;
-        for (int b = 0; b < B; ++b) {
-            db[b].q = hb[b].sigma * 2.0 * M_PI / (double)N;
-            db[b].shift = ((hb[b].shift % N) + N) % N;
-            logk[b] = stxmr_logk(db[b].q, N, logN);
-            const double aq = fabs(db[b].q);
-            const double km = aq > 0.0 ? ceil((logk[b] < logN ? STXMR_U : 14.5) / aq) + (logk[b] < logN ? 1.0 : 2.0) : (double)N;
-            db[b].kmax = km < (double)N ? (long long)km : (long long)N;
-        }
-        for (int lk = 0; lk <= logN; ++lk)
-            for (int b = 0; b < B; ++b) if (logk[b] == lk) ids.push_back(b);
-        stage_to_device(d_bands, db.data(), sizeof(DevStxBand) * (size_t)B, st);
-        stage_to_device(d_ids, ids.data(), sizeof(int) * (size_t)B, st);
+int qi_stx_multirate(const void* sig, int64_t C, int64_t N, int64_t stride, const QiStxBand* bands, int B, void* out_tfr,
+                     void* out_power, void* ws, size_t ws_bytes, void* stream) {
+    if (!sig || !bands || !ws || C <= 0 || C > 65535 || N <= 0 || B <= 0 || stride < N || (!out_tfr && !out_power)) return QI_ERR_ARG;
+    if ((N & (N - 1)) || N < 2 * qi::CWTF_TILE) return QI_ERR_ARG;
+    if (N > (1ll << 30)) return QI_ERR_UNSUPPORTED;
+    return qi::stx_multirate_impl(sig, C, N, stride, bands, B, out_tfr, out_power, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
 
-        CwtGeom geo;
-        geo.n_points = N; geo.n_channels = C; geo.n_bands = B; geo.logL = logN;
-        geo.conv_mode = QI_CONV_LINEAR_SAME; geo.fs = 0; geo.centre_idx = 0; geo.half_shift = 0; geo.d_min = 0; geo.d_max = 0;
-        const FftPlan plan = make_plan(logN, (int)sizeof(cplx<T>));
-        const T one = (T)1;
-        prof_set_category(QI_CAT_FFT_FWD);
-        for (int p = 0; p < plan.npass; ++p) {
-            DstComplex<T> d{spec, N, one};
-            if (p == 0) { SrcRealPad<T> s{static_cast<const T*>(sig), stride, N}; launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st); }
-            else { SrcComplex<T> s{spec, N}; launch_pass<T, FFT_FWD>(plan, p, C, s, d, 0, st); }
-        }
-        // interpolator tables of every decimation in use: one launch
-        unsigned need_mask = 0;
-        for (int b = 0; b < B; ++b) if (logk[b] < logN) need_mask |= 1u << (logN - logk[b]);
-        if (need_mask) {
-            prof_set_category(QI_CAT_OTHER);
-            dim3 cgrid((unsigned)((STXMR_TAPS << STXMR_MAX_LOGD) / 256), (unsigned)(STXMR_MAX_LOGD + 1));
-            QI_LAUNCH((stxmr_coef_kernel), cgrid, dim3(256), 0, st, coef, need_mask, 1.0 / stxmr_bessel_i0(STXMR_BETA));
-        }
-        // decimated groups
-        size_t pos = 0;
-        while (pos < ids.size()) {
-            const int lk = logk[ids[pos]];
-            size_t end = pos;
-            while (end < ids.size() && logk[ids[end]] == lk) ++end;
-            const int g = (int)(end - pos);
-            if (lk < logN) {
-                const int logD = logN - lk;
-                float* cf = coef + (size_t)logD * STXMR_TAPS * (1u << STXMR_MAX_LOGD);
-                const FftPlan pk = make_plan(lk, (int)sizeof(cplx<T>));
-                const i64 K = 1ll << lk;
-                for (i64 sub = 0; sub < g; ) {                         // grid.y limit: chunks of bands
-                    i64 gs = g - sub;
-                    while (gs * C > 65535) --gs;
-                    const i64 nb = gs * C;
-                    SrcStxDec s1{spec, d_bands, d_ids + pos + sub, (int)C, logN, lk};
-                    for (int p = pk.npass - 1; p >= 0; --p) {
-                        const bool first = (p == pk.npass - 1), last = (p == 0);
-                        SrcComplex<T> s2{work, K};
-                        DstComplex<T> dw{work, K, one}, dd{dec, K, one};
-                        prof_set_category(first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID);
-                        if (first && last) launch_pass<T, FFT_INV>(pk, p, nb, s1, dd, 0, st);
-                        else if (first) launch_pass<T, FFT_INV>(pk, p, nb, s1, dw, 0, st);
-                        else if (last) launch_pass<T, FFT_INV>(pk, p, nb, s2, dd, 0, st);
-                        else launch_pass<T, FFT_INV>(pk, p, nb, s2, dw, 0, st);
-                    }
-                    prof_set_category(QI_CAT_INV_LAST);
-                    dim3 grid((unsigned)((N + STXMR_SPAN * STXMR_TILE - 1) / (STXMR_SPAN * STXMR_TILE)), (unsigned)gs, (unsigned)C);
-                    QI_LAUNCH((stxmr_interp_kernel), grid, dim3(256), 0, st, (const cplx<T>*)dec, (const int*)(d_ids + pos + sub), (int)C, B,
-                              logN, logD, (const float*)cf, static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p));
-                    sub += gs;
-                }
-            } else {
-                // exact bands: the two full-length passes, over maximal runs of consecutive band indices
-                size_t r0 = pos;
-                while (r0 < end) {
-                    size_t r1 = r0 + 1;
-                    while (r1 < end && ids[r1] == ids[r1 - 1] + 1 && (i64)(r1 - r0) < lo.gx) ++r1;
-                    const int band0 = ids[r0], gr = (int)(r1 - r0);
-                    const i64 nb = (i64)gr * C;
-                    for (int p = plan.npass - 1; p >= 0; --p) {
-                        const bool first = (p == plan.npass - 1), last = (p == 0);
-                        SrcStxSpec<T> s1{spec, d_bands, band0, geo};
-                        SrcComplex<T> s2{work, N};
-                        DstComplex<T> d1{work, N, one};
-                        DstCwtOut<T> d2{static_cast<cplx<T>*>(out_c), static_cast<T*>(out_p), nullptr, band0, geo, 0.0};
-                        prof_set_category(last ? QI_CAT_INV_LAST : (first ? QI_CAT_INV_FIRST : QI_CAT_INV_MID));
-                        if (first && last) launch_pass<T, FFT_INV>(plan, p, nb, s1, d2, 256, st);
-                        else if (first) launch_pass<T, FFT_INV>(plan, p, nb, s1, d1, 0, st);
-                        else if (last) launch_pass<T, FFT_INV>(plan, p, nb, s2, d2, 256, st);
-                        else launch_pass<T, FFT_INV>(plan, p, nb, s2, d1, 0, st);
-                    }
-                    r0 = r1;
-                }
-            }
-            pos = end;
-        }
-        prof_set_category(QI_CAT_OTHER);
-        return check_cuda("qi_stx_multirate");
-    }
+size_t qi_stx_windows_workspace_bytes(int B) { return B > 0 ? sizeof(qi::DevStxBand) * (size_t)B : 0; }
 
-    template <typename T>
-    static int stx_windows_impl(const QiStxBand* hb, int B, i64 N, void* out, void* ws, size_t ws_bytes, cudaStream_t st) {
-        if (ws_bytes < sizeof(DevStxBand) * (size_t)B) return QI_ERR_WORKSPACE;
-        DevStxBand* d_bands = static_cast<DevStxBand*>(ws);
-        upload_stx_bands(hb, B, N, 1e300, d_bands, st);
-        dim3 grid((unsigned)((N + 255) / 256), (unsigned)B);
-        QI_LAUNCH((stx_windows_kernel<T>), grid, dim3(256), 0, st, d_bands, N, static_cast<cplx<T>*>(out));
-        return check_cuda("qi_stx_windows");
-    }
+int qi_stx_windows(const QiStxBand* bands, int B, int64_t N, int dtype, void* out, void* ws, size_t ws_bytes, void* stream) {
+    if (!bands || !out || !ws || B <= 0 || N <= 0) return QI_ERR_ARG;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (dtype == QI_F32) return qi::stx_windows_impl<float>(bands, B, N, out, ws, ws_bytes, st);
+    if (dtype == QI_F64) return qi::stx_windows_impl<double>(bands, B, N, out, ws, ws_bytes, st);
+    return QI_ERR_ARG;
+}
 
-    }  // namespace qi
-
-    extern "C" {
-
-    size_t qi_stx_workspace_bytes(int64_t C, int64_t N, int B, int group, int dtype) {
-        if (C <= 0 || N <= 0 || B <= 0) return 0;
-        if (group < 0) group = -group;
-        return dtype == QI_F32 ? qi::stx_layout<float>(C, N, B, group).total : qi::stx_layout<double>(C, N, B, group).total;
-    }
-
-    int qi_stx_fft(const void* sig, int64_t C, int64_t N, int64_t stride, const QiStxBand* bands, int B, int dtype,
-                   void* out_tfr, void* out_power, double* band_sum, void* ws, size_t ws_bytes, int group, void* stream) {
-        if (!sig || !bands || !ws || C <= 0 || N <= 0 || B <= 0 || stride < N) return QI_ERR_ARG;
-        if (N & (N - 1)) return QI_ERR_ARG;
-        if (N > (1ll << 30)) return QI_ERR_UNSUPPORTED;
-        cudaStream_t st = static_cast<cudaStream_t>(stream);
-        const bool fast = group >= 0;                  // a negative bands_per_group keeps every band on the full-length passes
-        if (group < 0) group = -group;
-        if (dtype == QI_F32) return qi::stx_fft_impl<float>(sig, C, N, stride, bands, B, out_tfr, out_power, band_sum, ws, ws_bytes, group, st, fast);
-        if (dtype == QI_F64) return qi::stx_fft_impl<double>(sig, C, N, stride, bands, B, out_tfr, out_power, band_sum, ws, ws_bytes, group, st, fast);
-        return QI_ERR_ARG;
-    }
-
-    size_t qi_stx_multirate_workspace_bytes(int64_t C, int64_t N, const QiStxBand* bands, int B) {
-        if (C <= 0 || N < qi::STXMR_TILE * 2 || (N & (N - 1)) || B <= 0 || !bands) return 0;
-        return qi::stxmr_layout(C, N, bands, B).total;
-    }
-
-    int qi_stx_multirate(const void* sig, int64_t C, int64_t N, int64_t stride, const QiStxBand* bands, int B, void* out_tfr,
-                         void* out_power, void* ws, size_t ws_bytes, void* stream) {
-        if (!sig || !bands || !ws || C <= 0 || C > 65535 || N <= 0 || B <= 0 || stride < N || (!out_tfr && !out_power)) return QI_ERR_ARG;
-        if ((N & (N - 1)) || N < qi::STXMR_TILE * 2) return QI_ERR_ARG;
-        if (N > (1ll << 30)) return QI_ERR_UNSUPPORTED;
-        return qi::stx_multirate_impl(sig, C, N, stride, bands, B, out_tfr, out_power, ws, ws_bytes, static_cast<cudaStream_t>(stream));
-    }
-
-    size_t qi_stx_windows_workspace_bytes(int B) { return B > 0 ? sizeof(qi::DevStxBand) * (size_t)B : 0; }
-
-    int qi_stx_windows(const QiStxBand* bands, int B, int64_t N, int dtype, void* out, void* ws, size_t ws_bytes, void* stream) {
-        if (!bands || !out || !ws || B <= 0 || N <= 0) return QI_ERR_ARG;
-        cudaStream_t st = static_cast<cudaStream_t>(stream);
-        if (dtype == QI_F32) return qi::stx_windows_impl<float>(bands, B, N, out, ws, ws_bytes, st);
-        if (dtype == QI_F64) return qi::stx_windows_impl<double>(bands, B, N, out, ws, ws_bytes, st);
-        return QI_ERR_ARG;
-    }
-
-    }  // extern "C"
+}  // extern "C"
