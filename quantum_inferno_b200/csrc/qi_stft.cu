@@ -4,7 +4,8 @@
 // zero-extended) record straight into shared memory, two real frames packed into one complex column,
 // the per-frame mean removed, the periodic window applied, one radix-8 tile FFT run, the two spectra
 // separated with the Hermitian split and the one-sided bins stored with time as the fastest axis (the
-// layout scipy returns).  Replaces scipy.signal.stft / welch as called by
+// layout scipy returns).  Frames too long for one CTA take multi-pass FFTs of frame pairs instead (the long-frame route
+// below).  Replaces scipy.signal.stft / welch as called by
 // quantum_inferno/styx_fft.py:175-187, :215-227, :254-266, and scipy.signal.ShortTimeFFT.stft_detrend / spectrogram /
 // istft as called by quantum_inferno/utilities/short_time_fft.py:64-175.
 #include "qi_fft.cuh"
@@ -258,29 +259,201 @@ stft_kernel(const T* __restrict__ sig, const T* __restrict__ window, StftGeom g0
     }
 }
 
+// dynamic shared memory of stft_kernel with tc tiles of nfft points
+template <typename T> static size_t stft_tile_smem(int nfft, int tc) {
+    return ((size_t)stft_tile_pitch<T>(nfft) * tc + nfft) * sizeof(cplx<T>) + 2 * tc * sizeof(T) +
+           (2 * tc + 16) * sizeof(double) + 64;
+}
+// QI_STFT_TILE_MAX_NFFT > 0 sends every longer frame to the long-frame route below (tools/stft_long_probe.py builds such a
+// variant to time both routes at the same size); 0: the shared-memory budget alone decides
+#ifndef QI_STFT_TILE_MAX_NFFT
+#define QI_STFT_TILE_MAX_NFFT 0
+#endif
+// tiles per CTA of stft_kernel, or 0 when one frame does not fit a CTA: <= ~100 KB per CTA so that two CTAs (2 x 512
+// threads) share an SM; one big CTA for long FFTs
+template <typename T> static int stft_tile_columns(int nfft) {
+    if (QI_STFT_TILE_MAX_NFFT > 0 && nfft > QI_STFT_TILE_MAX_NFFT) return 0;
+    size_t budget = StftLaunch<T>::budget;
+    int TC = 16;
+    while (TC > 2 && stft_tile_smem<T>(nfft, TC) > budget) TC >>= 1;
+    if (stft_tile_smem<T>(nfft, TC) > budget) {
+        budget = 200 * 1024;
+        while (TC > 1 && stft_tile_smem<T>(nfft, TC) > budget) TC >>= 1;
+    }
+    return stft_tile_smem<T>(nfft, TC) > budget ? 0 : TC;
+}
+
+// ---------------------------------------------------------------- frames longer than one CTA's shared memory
+// The frame lengths stft_kernel / istft_frames_kernel refuse (float32 nfft >= 2^14, float64 >= 2^13) take the multi-pass
+// FFT of qi_fft.cuh with the same two-real-frames-per-complex-row packing.  Frame pairs are processed in chunks of npc
+// pairs per channel: batch row b = chan * npc + (p - p0) holds pair p (frames 2p, 2p + 1), its spectrum in bit-reversed
+// order, nfft elements per row.
+//   forward: stft_long_means_kernel (fp64 frame sums) -> forward passes whose first pass gathers (x - mean) * window
+//            (SrcStftPair) -> stft_split_kernel (Hermitian split, roll phase, scale, scipy's layout, Welch sums)
+//   inverse: istft_gather_kernel (undo the roll, Hermitian-completed Z = Xa + i Xb) -> inverse passes whose last pass
+//            applies the dual window (DstIstftPair) -> istft_ola_kernel as for the tile route
+// The split and the gather work on aligned blocks of P = STFT_LONG_P storage positions: block brev(c) holds the bins
+// c + j nfft / P (j < P), and the Hermitian partners nfft - k of those bins fill the block of residue nfft / P - c.  A CTA
+// takes one such block pair for P consecutive frame pairs: contiguous reads along the positions, runs of 2 P consecutive
+// frames in the [C, nfft/2+1, n_frames] store.
+constexpr int STFT_LONG_LOGP = 5, STFT_LONG_P = 1 << STFT_LONG_LOGP;   // positions per block = frame pairs per CTA
+
+// bytes of workspace per frame pair and channel: the pair spectrum and the two frame means
+template <typename T> static size_t stft_long_pair_bytes(int nfft) { return (size_t)nfft * sizeof(cplx<T>) + 2 * sizeof(T); }
+
+// mean of frame f0 + blockIdx.x over its nperseg samples of the zero-extended record, summed in fp64 and rounded to T as
+// stft_kernel does; frames >= n_frames get 0.  means[chan][gridDim.x]
+template <typename T>
+__global__ void __launch_bounds__(256)
+stft_long_means_kernel(const T* __restrict__ sig, i64 sig_stride, i64 n_points, i64 n_frames, i64 f0, int nperseg,
+                       int hop, int pad_left, T* __restrict__ means) {
+    __shared__ double scratch[32];
+    const i64 chan = blockIdx.y, f = f0 + blockIdx.x;
+    const T* x = sig + chan * sig_stride;
+    double s0 = 0.0, s1 = 0.0;
+    if (f < n_frames) {
+        const i64 start = f * hop - pad_left;
+        const i64 lo = start > 0 ? start : 0, hi = start + nperseg < n_points ? start + nperseg : n_points;
+        i64 i = lo + threadIdx.x;
+        for (; i + (i64)blockDim.x < hi; i += 2 * (i64)blockDim.x) { s0 += (double)x[i]; s1 += (double)x[i + blockDim.x]; }
+        if (i < hi) s0 += (double)x[i];
+    }
+    const double s = block_sum(s0 + s1, scratch);
+    if (threadIdx.x == 0) means[chan * gridDim.x + blockIdx.x] = (T)(s / (double)nperseg);
+}
+
+// first forward pass: element e of row b = ((x[fa hop + e - pad_left] - mean_a) w[e], (x[fb hop + ...] - mean_b) w[e]),
+// the record zero-extended, the frame zero-padded from nperseg to nfft, a frame >= n_frames all zero
+template <typename T> struct SrcStftPair {
+    const T* sig; const T* window; const T* means;       // means [rows][2], or NULL without detrend
+    i64 sig_stride, n_points, n_frames, p0;
+    int npc, nperseg, hop, pad_left;
+    QI_DEV cplx<T> load(i64 b, i64 e) const {
+        if (e >= nperseg) return mk<T>((T)0, (T)0);
+        const unsigned bu = (unsigned)b;                  // b < 65536 (grid.y)
+        const i64 chan = bu / (unsigned)npc, fa = 2 * (p0 + bu % (unsigned)npc);
+        const T* x = sig + chan * sig_stride;
+        const i64 pa = fa * hop + e - pad_left, pb = pa + hop;
+        T va = fa < n_frames && pa >= 0 && pa < n_points ? x[pa] : (T)0;
+        T vb = fa + 1 < n_frames && pb >= 0 && pb < n_points ? x[pb] : (T)0;
+        if (means) { va -= means[2 * b]; vb -= means[2 * b + 1]; }
+        const T w = window[e];
+        return mk<T>(va * w, vb * w);
+    }
+};
+
+// shared-memory slot of storage offset i of block q (0: residue c, 1: its partner) for frame pair t
+QI_HD int stft_long_slot(int q, int t, int i) { return (q * STFT_LONG_P + t) * (STFT_LONG_P + 1) + i; }
+
+// Hermitian split of the pair spectra of one chunk (buf [C * npc][nfft], bit-reversed) into the one-sided bins of both
+// frames, times the roll phase and the scale: out [C, nfft/2+1, n_frames] and / or psd_acc [C, nfft/2+1] += |X_k|^2.
+// grid = (nfft / (2 LP) + 1 block pairs, ceil(npc / LP), C); 256 threads; one warp per bin, lanes along the frame pairs.
+template <typename T>
+__global__ void __launch_bounds__(256)
+stft_split_kernel(const cplx<T>* __restrict__ buf, int logL, int npc, i64 p0, i64 n_frames, int roll, T sc,
+                  cplx<T>* __restrict__ out, double* __restrict__ psd_acc) {
+    QI_DYN_SMEM(smem_raw);
+    constexpr int P = STFT_LONG_P, logP = STFT_LONG_LOGP;
+    cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
+    const int L = 1 << logL, nblk = L >> logP, K = (L >> 1) + 1;
+    const int c = blockIdx.x, c2 = (nblk - c) & (nblk - 1), nb = c2 == c ? 1 : 2;
+    const int t0 = blockIdx.y * P, ntp = npc - t0 < P ? npc - t0 : P;
+    const i64 chan = blockIdx.z;
+    const cplx<T>* rows = buf + (chan * npc + t0) * (i64)L;
+    for (int idx = threadIdx.x; idx < nb * P * P; idx += blockDim.x) {     // lanes along the positions of one row
+        const int i = idx & (P - 1), t = (idx >> logP) & (P - 1), q = idx >> (2 * logP);
+        if (t < ntp) s[stft_long_slot(q, t, i)] = rows[(i64)t * L + brev_bits((unsigned)(q ? c2 : c), logL) + i];
+    }
+    __syncthreads();
+    const int t = threadIdx.x & 31;
+    const i64 fa = 2 * (p0 + t0 + t);
+    for (int slot = threadIdx.x >> 5; slot < nb * P; slot += blockDim.x >> 5) {
+        const int q = slot >> logP, j = slot & (P - 1);
+        const int k = (q ? c2 : c) + (j << (logL - logP));
+        if (k > (L >> 1)) continue;                                       // the partner's warp has it
+        const int k2 = (L - k) & (L - 1);
+        const int q2 = (k2 & (nblk - 1)) == c ? 0 : 1;
+        cplx<T> z1 = mk<T>((T)0, (T)0), z2 = z1;
+        if (t < ntp) {
+            z1 = s[stft_long_slot(q, t, (int)brev_bits((unsigned)j, logP))];
+            z2 = s[stft_long_slot(q2, t, (int)brev_bits((unsigned)(k2 >> (logL - logP)), logP))];
+        }
+        cplx<T> xa = mk<T>((T)0.5 * (z1.re + z2.re), (T)0.5 * (z1.im - z2.im));
+        cplx<T> xb = mk<T>((T)0.5 * (z1.im + z2.im), (T)-0.5 * (z1.re - z2.re));
+        if (roll) {
+            const cplx<T> ph = unit_root<T>((unsigned long long)(((i64)k * roll) & (L - 1)), logL);
+            xa = xa * ph; xb = xb * ph;
+        }
+        if (out && t < ntp) {
+            cplx<T>* o = out + (chan * K + k) * n_frames + fa;
+            if (fa < n_frames) o[0] = xa * sc;
+            if (fa + 1 < n_frames) o[1] = xb * sc;
+        }
+        if (psd_acc) {
+            double pw = 0.0;
+            if (t < ntp && fa < n_frames) pw += (double)norm2(xa);
+            if (t < ntp && fa + 1 < n_frames) pw += (double)norm2(xb);
+            pw = warp_sum(pw);
+            if (t == 0) atomicAdd(&psd_acc[chan * K + k], pw);
+        }
+    }
+}
+
+template <typename T>
+static int stft_long(const T* sig, i64 C, i64 n_points, i64 stride, const T* window, int nperseg, int hop, int logL,
+                     i64 n_frames, int pad_left, double scale, int detrend, int roll, cplx<T>* out, double* psd_acc,
+                     void* ws, size_t ws_bytes, cudaStream_t st) {
+    const int L = 1 << logL;
+    const size_t per_pair = stft_long_pair_bytes<T>(L) * (size_t)C;
+    if (ws_bytes < per_pair) return QI_ERR_WORKSPACE;
+    if (reinterpret_cast<uintptr_t>(ws) % sizeof(cplx<T>)) return QI_ERR_ARG;
+    const i64 npairs = (n_frames + 1) / 2;
+    i64 npc = (i64)(ws_bytes / per_pair);
+    if (npc > 65535 / C) npc = 65535 / C;                 // batch rows per launch: grid.y
+    if (npc > npairs) npc = npairs;
+    cplx<T>* buf = static_cast<cplx<T>*>(ws);
+    T* means = reinterpret_cast<T*>(buf + (size_t)C * npc * L);
+    const FftPlan plan = make_plan(logL, (int)sizeof(cplx<T>));
+    const int nblk = L >> STFT_LONG_LOGP;
+    const size_t split_smem = (size_t)2 * STFT_LONG_P * (STFT_LONG_P + 1) * sizeof(cplx<T>);
+    if (psd_acc) cudaMemsetAsync(psd_acc, 0, sizeof(double) * (size_t)C * (L / 2 + 1), st);
+    for (i64 p0 = 0; p0 < npairs; p0 += npc) {
+        const int n = (int)(npairs - p0 < npc ? npairs - p0 : npc);
+        prof_set_category(QI_CAT_STFT);
+        if (detrend)
+            QI_LAUNCH((stft_long_means_kernel<T>), dim3((unsigned)(2 * n), (unsigned)C), dim3(256), 0, st, sig, stride,
+                      n_points, n_frames, 2 * p0, nperseg, hop, pad_left, means);
+        const SrcStftPair<T> src{sig, window, detrend ? means : nullptr, stride, n_points, n_frames, p0, n, nperseg, hop,
+                                 pad_left};
+        forward_passes<T>(plan, C * n, src, buf, L, st);
+        QI_LAUNCH((stft_split_kernel<T>), dim3((unsigned)(nblk / 2 + 1), (unsigned)((n + STFT_LONG_P - 1) / STFT_LONG_P),
+                  (unsigned)C), dim3(256), split_smem, st, buf, logL, n, p0, n_frames, roll, (T)scale, out, psd_acc);
+    }
+    return check_cuda("qi_stft");
+}
+
 template <typename T>
 static int stft_impl(const void* sig, i64 C, i64 n_points, i64 stride, const void* window, int nperseg, int hop,
                      int nfft, i64 n_frames, int pad_left, double scale, int detrend, int roll, void* out,
-                     double* psd_acc, cudaStream_t st) {
+                     double* psd_acc, void* ws, size_t ws_bytes, cudaStream_t st) {
     int logF = 0;
     while ((1 << logF) < nfft) ++logF;
     if ((1 << logF) != nfft) return QI_ERR_ARG;
-    // <= ~100 KB per CTA so that two CTAs (2 x 512 threads) share an SM; fall back to one big CTA for long FFTs
-    size_t budget = StftLaunch<T>::budget;
-    int TC = 16;
-    auto need = [&](int tc) { return ((size_t)stft_tile_pitch<T>(nfft) * tc + nfft) * sizeof(cplx<T>) + 2 * tc * sizeof(T) + (2 * tc + 16) * sizeof(double) + 64; };
-    while (TC > 2 && need(TC) > budget) TC >>= 1;
-    if (need(TC) > budget) { budget = 200 * 1024; while (TC > 1 && need(TC) > budget) TC >>= 1; }
-    if (need(TC) > budget) return QI_ERR_UNSUPPORTED;
+    const int TC = stft_tile_columns<T>(nfft);
+    if (TC == 0 && !ws) return QI_ERR_UNSUPPORTED;
+    if (C > 65535) return QI_ERR_UNSUPPORTED;
+    if (TC == 0)
+        return stft_long<T>(static_cast<const T*>(sig), C, n_points, stride, static_cast<const T*>(window), nperseg, hop,
+                            logF, n_frames, pad_left, scale, detrend, ((roll % nfft) + nfft) % nfft,
+                            static_cast<cplx<T>*>(out), psd_acc, ws, ws_bytes, st);
     // the psd reduction uses shuffles across the TC lanes of one k: needs TC | 32 (true: power of two <= 16)
     StftGeom g;
     g.n_points = n_points; g.sig_stride = stride; g.n_frames = n_frames;
     g.nperseg = nperseg; g.hop = hop; g.logF = logF; g.pad_left = pad_left; g.TC = TC; g.detrend = detrend;
     g.roll = ((roll % nfft) + nfft) % nfft;
     g.scale = scale;
-    if (C > 65535) return QI_ERR_UNSUPPORTED;
     dim3 grid((unsigned)((n_frames + 2 * TC - 1) / (2 * TC)), (unsigned)C);
-    const size_t smem = need(TC);
+    const size_t smem = stft_tile_smem<T>(nfft, TC);
     if (psd_acc) cudaMemsetAsync(psd_acc, 0, sizeof(double) * (size_t)C * (nfft / 2 + 1), st);
     prof_set_category(QI_CAT_STFT);
     int logTC = 0;
@@ -408,6 +581,114 @@ istft_ola_kernel(const T* __restrict__ slices, IstftGeom g, T* __restrict__ out)
     out[chan * g.n_out + i] = acc;
 }
 
+// dynamic shared memory of istft_frames_kernel with tc columns, and its columns per CTA (0: the frame does not fit)
+static size_t istft_tile_smem(int nfft, int tc, size_t elem_bytes) { return (size_t)nfft * (tc + 2) * elem_bytes + 64; }
+template <typename T> static int istft_tile_columns(int nfft) {
+    size_t budget = 100 * 1024;
+    int TC = 16;
+    while (TC > 2 && istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) TC >>= 1;
+    if (istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) {
+        budget = 200 * 1024;
+        while (TC > 1 && istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) TC >>= 1;
+    }
+    return istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget ? 0 : TC;
+}
+
+// Long frames: Hermitian-completed pair spectra Z = Xa + i Xb of one chunk (S [C, nfft/2+1, P] -> buf [C * npc][nfft],
+// bit-reversed rows), the roll undone; the imaginary parts of bins 0 and nfft/2 dropped as irfft does.  Same grid and
+// block pairing as stft_split_kernel.
+template <typename T>
+__global__ void __launch_bounds__(256)
+istft_gather_kernel(const cplx<T>* __restrict__ S, int logL, int npc, i64 p0, i64 n_frames, int roll,
+                    cplx<T>* __restrict__ buf) {
+    QI_DYN_SMEM(smem_raw);
+    constexpr int P = STFT_LONG_P, logP = STFT_LONG_LOGP;
+    cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
+    const int L = 1 << logL, nblk = L >> logP, K = (L >> 1) + 1;
+    const int c = blockIdx.x, c2 = (nblk - c) & (nblk - 1), nb = c2 == c ? 1 : 2;
+    const int t0 = blockIdx.y * P, ntp = npc - t0 < P ? npc - t0 : P;
+    const i64 chan = blockIdx.z;
+    const int t = threadIdx.x & 31;
+    const i64 fa = 2 * (p0 + t0 + t);
+    for (int slot = threadIdx.x >> 5; slot < nb * P; slot += blockDim.x >> 5) {
+        const int q = slot >> logP, j = slot & (P - 1);
+        const int k = (q ? c2 : c) + (j << (logL - logP));
+        if (k > (L >> 1) || t >= ntp) continue;                          // bins above nfft/2: the partner's warp
+        const int k2 = (L - k) & (L - 1);
+        const int q2 = (k2 & (nblk - 1)) == c ? 0 : 1;
+        cplx<T> xa = mk<T>((T)0, (T)0), xb = xa;
+        if (fa < n_frames) xa = S[(chan * K + k) * n_frames + fa];
+        if (fa + 1 < n_frames) xb = S[(chan * K + k) * n_frames + fa + 1];
+        if (roll) {
+            const cplx<T> ph = conj(unit_root<T>((unsigned long long)(((i64)k * roll) & (L - 1)), logL));
+            xa = xa * ph; xb = xb * ph;
+        }
+        const int i1 = (int)brev_bits((unsigned)j, logP);
+        if (k == 0 || k == (L >> 1)) {
+            s[stft_long_slot(q, t, i1)] = mk<T>(xa.re, xb.re);
+        } else {
+            s[stft_long_slot(q, t, i1)] = mk<T>(xa.re - xb.im, xa.im + xb.re);
+            s[stft_long_slot(q2, t, (int)brev_bits((unsigned)(k2 >> (logL - logP)), logP))] = mk<T>(xa.re + xb.im, xb.re - xa.im);
+        }
+    }
+    __syncthreads();
+    cplx<T>* rows = buf + (chan * npc + t0) * (i64)L;
+    for (int idx = threadIdx.x; idx < nb * P * P; idx += blockDim.x) {     // lanes along the positions of one row
+        const int i = idx & (P - 1), tt = (idx >> logP) & (P - 1), q = idx >> (2 * logP);
+        if (tt < ntp) rows[(i64)tt * L + brev_bits((unsigned)(q ? c2 : c), logL) + i] = s[stft_long_slot(q, tt, i)];
+    }
+}
+
+// last inverse pass of the long route: sample n < nperseg of row b's two frames, times dual_win[n] / nfft, into the
+// slices [C][n_frames][nperseg] of istft_frames_kernel
+template <typename T> struct DstIstftPair {
+    T* slices; const T* dual_win;
+    i64 n_frames, p0;
+    int npc, nperseg;
+    T inv;
+    QI_DEV void store(i64 b, i64 n, cplx<T> v) const {
+        if (n >= nperseg) return;
+        const unsigned bu = (unsigned)b;                  // b < 65536 (grid.y)
+        const i64 chan = bu / (unsigned)npc, fa = 2 * (p0 + bu % (unsigned)npc);
+        const T w = dual_win[n] * inv;
+        T* o = slices + (chan * n_frames + fa) * nperseg + n;
+        o[0] = v.re * w;
+        if (fa + 1 < n_frames) o[nperseg] = v.im * w;
+    }
+    QI_DEV void finish(i64, unsigned char*) const {}
+};
+
+// long-route workspace: the slices (rounded up to 256 bytes), then the pair spectra of one chunk
+static i64 istft_long_pairs_per_chunk(i64 C, i64 n_frames) {
+    const i64 npairs = (n_frames + 1) / 2, cap = 65535 / C;
+    return npairs < cap ? npairs : cap;
+}
+static size_t istft_slices_bytes(i64 C, i64 n_frames, int nperseg, size_t real_bytes) {
+    return (size_t)C * (size_t)n_frames * (size_t)nperseg * real_bytes;
+}
+
+template <typename T>
+static void istft_long_slices(const cplx<T>* S, i64 C, i64 P, const T* dual_win, int nperseg, int logL, int roll, T* slices,
+                              cudaStream_t st) {
+    const int L = 1 << logL;
+    const i64 npairs = (P + 1) / 2, npc = istft_long_pairs_per_chunk(C, P);
+    cplx<T>* buf = reinterpret_cast<cplx<T>*>(reinterpret_cast<unsigned char*>(slices) +
+                                              (istft_slices_bytes(C, P, nperseg, sizeof(T)) + 255) / 256 * 256);
+    const FftPlan plan = make_plan(logL, (int)sizeof(cplx<T>));
+    const int nblk = L >> STFT_LONG_LOGP;
+    const size_t smem = (size_t)2 * STFT_LONG_P * (STFT_LONG_P + 1) * sizeof(cplx<T>);
+    const T inv = (T)(1.0 / (double)L);
+    for (i64 p0 = 0; p0 < npairs; p0 += npc) {
+        const int n = (int)(npairs - p0 < npc ? npairs - p0 : npc);
+        prof_set_category(QI_CAT_STFT);
+        QI_LAUNCH((istft_gather_kernel<T>), dim3((unsigned)(nblk / 2 + 1), (unsigned)((n + STFT_LONG_P - 1) / STFT_LONG_P),
+                  (unsigned)C), dim3(256), smem, st, S, logL, n, p0, P, roll, buf);
+        const DstIstftPair<T> dst{slices, dual_win, P, p0, n, nperseg, inv};
+        inverse_passes<T>(plan, C * n, SrcComplex<T>{buf, L}, dst, 0, false, buf, L, st);
+    }
+    prof_set_category(QI_CAT_STFT);
+}
+
 template <typename T>
 static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int nperseg, int hop, int nfft, int roll,
                       i64 first_start, i64 frame_lo, i64 frame_hi, i64 k0, i64 n_out, void* out, void* ws,
@@ -415,24 +696,25 @@ static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int npe
     int logF = 0;
     while ((1 << logF) < nfft) ++logF;
     if ((1 << logF) != nfft) return QI_ERR_ARG;
-    size_t budget = 100 * 1024;
-    int TC = 16;
-    auto need = [&](int tc) { return ((size_t)nfft * (tc + 2)) * sizeof(cplx<T>) + 64; };
-    while (TC > 2 && need(TC) > budget) TC >>= 1;
-    if (need(TC) > budget) { budget = 200 * 1024; while (TC > 1 && need(TC) > budget) TC >>= 1; }
-    if (need(TC) > budget) return QI_ERR_UNSUPPORTED;
+    const int TC = istft_tile_columns<T>(nfft);
     if (C > 65535) return QI_ERR_UNSUPPORTED;
     IstftGeom g;
     g.n_frames = P; g.first_start = first_start; g.frame_lo = frame_lo; g.frame_hi = frame_hi; g.k0 = k0; g.n_out = n_out;
     g.nperseg = nperseg; g.hop = hop; g.logF = logF; g.TC = TC; g.roll = ((roll % nfft) + nfft) % nfft;
-    const size_t smem = need(TC);
+    if (TC == 0) {
+        if (reinterpret_cast<uintptr_t>(ws) % sizeof(cplx<T>)) return QI_ERR_ARG;
+        istft_long_slices<T>(static_cast<const cplx<T>*>(S), C, P, static_cast<const T*>(dual_win), nperseg, logF, g.roll,
+                             static_cast<T*>(ws), st);
+    } else {
+        const size_t smem = istft_tile_smem(nfft, TC, sizeof(cplx<T>));
 #ifndef QI_EMUL
-    cudaFuncSetAttribute(istft_frames_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(istft_frames_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 #endif
-    prof_set_category(QI_CAT_STFT);
-    dim3 grid((unsigned)((P + 2 * TC - 1) / (2 * TC)), (unsigned)C);
-    QI_LAUNCH((istft_frames_kernel<T>), grid, dim3(512), smem, st, static_cast<const cplx<T>*>(S),
-              static_cast<const T*>(dual_win), g, static_cast<T*>(ws));
+        prof_set_category(QI_CAT_STFT);
+        dim3 grid((unsigned)((P + 2 * TC - 1) / (2 * TC)), (unsigned)C);
+        QI_LAUNCH((istft_frames_kernel<T>), grid, dim3(512), smem, st, static_cast<const cplx<T>*>(S),
+                  static_cast<const T*>(dual_win), g, static_cast<T*>(ws));
+    }
     dim3 grid2((unsigned)((n_out + 255) / 256), (unsigned)C);
     QI_LAUNCH((istft_ola_kernel<T>), grid2, dim3(256), 0, st, static_cast<const T*>(ws), g, static_cast<T*>(out));
     return check_cuda("qi_istft");
@@ -440,9 +722,32 @@ static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int npe
 
 }  // namespace qi
 
+namespace {
+bool is_pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }
+// true when the tile kernels refuse this frame length in this dtype (the long-frame route takes it)
+bool long_frames(int nfft, int dtype, bool inverse) {
+    if (!is_pow2(nfft) || (dtype != QI_F32 && dtype != QI_F64)) return false;
+    if (inverse) return (dtype == QI_F64 ? qi::istft_tile_columns<double>(nfft) : qi::istft_tile_columns<float>(nfft)) == 0;
+    return (dtype == QI_F64 ? qi::stft_tile_columns<double>(nfft) : qi::stft_tile_columns<float>(nfft)) == 0;
+}
+}  // namespace
+
+extern "C" size_t qi_stft_workspace_bytes(int64_t C, int64_t n_frames, int nfft, int dtype) {
+    if (C <= 0 || n_frames <= 0 || !long_frames(nfft, dtype, false)) return 0;
+    const size_t per_pair = dtype == QI_F64 ? qi::stft_long_pair_bytes<double>(nfft) : qi::stft_long_pair_bytes<float>(nfft);
+    return (size_t)C * (size_t)((n_frames + 1) / 2) * per_pair;
+}
+
 extern "C" size_t qi_istft_workspace_bytes(int64_t C, int64_t n_frames, int nperseg, int dtype) {
     if (C <= 0 || n_frames <= 0 || nperseg <= 0) return 0;
-    return (size_t)C * (size_t)n_frames * (size_t)nperseg * (dtype == QI_F64 ? 8 : 4);
+    return qi::istft_slices_bytes(C, n_frames, nperseg, dtype == QI_F64 ? 8 : 4);
+}
+
+extern "C" size_t qi_istft_workspace_bytes_nfft(int64_t C, int64_t n_frames, int nperseg, int nfft, int dtype) {
+    const size_t slices = qi_istft_workspace_bytes(C, n_frames, nperseg, dtype);
+    if (slices == 0 || C > 65535 || !long_frames(nfft, dtype, true)) return slices;
+    return (slices + 255) / 256 * 256 +
+           (size_t)C * (size_t)qi::istft_long_pairs_per_chunk(C, n_frames) * (size_t)nfft * (dtype == QI_F64 ? 16 : 8);
 }
 
 extern "C" int qi_istft(const void* S, int64_t C, int64_t n_frames, const void* dual_win, int nperseg, int hop, int nfft,
@@ -451,7 +756,7 @@ extern "C" int qi_istft(const void* S, int64_t C, int64_t n_frames, const void* 
     if (!S || !dual_win || !out || !ws || C <= 0 || n_frames <= 0 || nperseg <= 0 || hop <= 0 || nfft < nperseg ||
         n_out <= 0 || frame_lo < 0 || frame_hi > n_frames || frame_lo >= frame_hi)
         return QI_ERR_ARG;
-    if (ws_bytes < qi_istft_workspace_bytes(C, n_frames, nperseg, dtype)) return QI_ERR_WORKSPACE;
+    if (ws_bytes < qi_istft_workspace_bytes_nfft(C, n_frames, nperseg, nfft, dtype)) return QI_ERR_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (dtype == QI_F32)
         return qi::istft_impl<float>(S, C, n_frames, dual_win, nperseg, hop, nfft, roll, first_start, frame_lo, frame_hi,
@@ -462,18 +767,26 @@ extern "C" int qi_istft(const void* S, int64_t C, int64_t n_frames, const void* 
     return QI_ERR_ARG;
 }
 
-extern "C" int qi_stft(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window, int nperseg,
-                       int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll, int dtype,
-                       void* out, double* psd_acc, void* stream) {
+extern "C" int qi_stft_ws(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window,
+                          int nperseg, int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend,
+                          int roll, int dtype, void* out, double* psd_acc, void* workspace, size_t workspace_bytes,
+                          void* stream) {
     if (!sig || !window || C <= 0 || n_points <= 0 || nperseg <= 0 || hop <= 0 || nfft < nperseg || n_frames <= 0)
         return QI_ERR_ARG;
     if (!out && !psd_acc) return QI_ERR_ARG;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (dtype == QI_F32)
         return qi::stft_impl<float>(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale,
-                                    detrend, roll, out, psd_acc, st);
+                                    detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
     if (dtype == QI_F64)
         return qi::stft_impl<double>(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale,
-                                     detrend, roll, out, psd_acc, st);
+                                     detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
     return QI_ERR_ARG;
+}
+
+extern "C" int qi_stft(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window, int nperseg,
+                       int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll, int dtype,
+                       void* out, double* psd_acc, void* stream) {
+    return qi_stft_ws(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale, detrend, roll,
+                      dtype, out, psd_acc, nullptr, 0, stream);
 }

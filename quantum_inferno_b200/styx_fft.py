@@ -6,7 +6,9 @@ The reference delegates to scipy.signal.stft / welch; here the frame gather, det
 scaling are one CUDA kernel (csrc/qi_stft.cu) with scipy's exact edge semantics: zero extension by
 nperseg//2 on both sides, zero padding to a whole number of hops, per-frame mean removal after the
 extension, DFT-even (periodic) window, scale 1/sum(window).  ``nfft`` must be a power of two (it always is
-through the *_pow2 defaults).  Keyword-only extra: ``dtype``.
+through the *_pow2 defaults).  Frames longer than one CTA's shared memory holds (float32 nfft > 8192, float64 > 4096)
+take multi-pass FFTs of frame pairs through a scratch buffer instead, with the same edge semantics.  Keyword-only
+extra: ``dtype``.
 
 The Butterworth pre-filters of the reference module (styx_fft.py:60-149: Tukey taper, ``scipy.signal.butter``,
 ``scipy.signal.filtfilt``) run on the device too: scipy designs the (b, a) taps and the steady-state initial
