@@ -19,7 +19,7 @@
 extern "C" {
 #endif
 
-#define QI_ABI_VERSION 4
+#define QI_ABI_VERSION 5
 
 /* dtype of the arithmetic and of every real/complex buffer in a call */
 #define QI_F32 0
@@ -198,22 +198,19 @@ int qi_stx_windows(const QiStxBand* bands, int n_bands, int64_t n_points, int dt
  *   roll    : the windowed, zero-padded segment is rotated left by `roll` samples before the transform, i.e. bin k is
  *             multiplied by exp(+2*pi*i*k*roll/nfft) (scipy.signal.ShortTimeFFT phase_shift, used through
  *             quantum_inferno/utilities/short_time_fft.py:54-58); 0 for scipy.signal.stft
- * A frame is transformed in one CTA's shared memory up to nfft = 8192 (float32) / 4096 (float64).  Longer frames take
- * multi-pass FFTs of frame pairs through a workspace (qi_stft_ws); qi_stft, which has none, returns
- * QI_ERR_UNSUPPORTED for them. */
+ * A frame is transformed in one CTA's shared memory up to nfft = 8192 (float32) / 4096 (float64) and needs no
+ * workspace (NULL, 0).  Longer frames take multi-pass FFTs of frame pairs through the workspace, in as many chunks as it
+ * takes: any workspace of at least one frame pair per channel (qi_stft_workspace_bytes with n_frames = 2) works, a
+ * smaller one is QI_ERR_WORKSPACE and NULL is QI_ERR_UNSUPPORTED.  The complex outputs do not depend on the chunk size,
+ * psd_acc only up to the order of its fp64 additions.
+ *   workspace: 256-byte aligned, or NULL */
 int qi_stft(const void* sig, int64_t n_channels, int64_t n_points, int64_t sig_stride, const void* window,
             int nperseg, int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll,
-            int dtype, void* out, double* psd_acc, void* stream);
+            int dtype, void* out, double* psd_acc, void* workspace, size_t workspace_bytes, void* stream);
 
-/* Workspace of qi_stft_ws: 0 for every nfft the one-CTA kernel takes; otherwise the bytes that transform all frames in
- * one chunk, n_channels * ceil(n_frames / 2) * (nfft complex values + 2 reals).  qi_stft_ws accepts any workspace of at
- * least one frame pair per channel (this function with n_frames = 2) and processes the frames in as many chunks as
- * that takes; the complex outputs do not depend on the chunk size, psd_acc only up to the order of its fp64 additions.
- * A smaller workspace is QI_ERR_WORKSPACE.  workspace: 256-byte aligned, or NULL (then as qi_stft). */
+/* Workspace of qi_stft that transforms all frames in one chunk: 0 for every nfft one CTA takes; otherwise
+ * n_channels * ceil(n_frames / 2) * (nfft complex values + 2 reals). */
 size_t qi_stft_workspace_bytes(int64_t n_channels, int64_t n_frames, int nfft, int dtype);
-int qi_stft_ws(const void* sig, int64_t n_channels, int64_t n_points, int64_t sig_stride, const void* window,
-               int nperseg, int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll,
-               int dtype, void* out, double* psd_acc, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Inverse STFT by overlap-add (scipy.signal.ShortTimeFFT.istft as called by
  * quantum_inferno/utilities/short_time_fft.py:106-134).
@@ -221,15 +218,15 @@ int qi_stft_ws(const void* sig, int64_t n_channels, int64_t n_points, int64_t si
  *   dual_win : real [nperseg] device pointer (canonical dual window; any scaling folded in)
  *   frame p covers output samples [first_start + p*hop, ... + nperseg); frames [frame_lo, frame_hi) are summed
  *   out      : real [n_channels, n_out] = samples k0 .. k0 + n_out - 1
- *   workspace: >= qi_istft_workspace_bytes_nfft, 256-byte aligned.  That is the windowed inverse transforms of all
- *              frames (qi_istft_workspace_bytes) for the frame lengths one CTA transforms (nfft <= 8192 float32 /
- *              4096 float64), and for longer frames those plus the pair spectra of up to 65535 frame pairs (multi-pass
- *              inverse FFTs). */
-size_t qi_istft_workspace_bytes(int64_t n_channels, int64_t n_frames, int nperseg, int dtype);
-size_t qi_istft_workspace_bytes_nfft(int64_t n_channels, int64_t n_frames, int nperseg, int nfft, int dtype);
+ *   workspace: >= qi_istft_workspace_bytes, 256-byte aligned */
 int qi_istft(const void* S, int64_t n_channels, int64_t n_frames, const void* dual_win, int nperseg, int hop, int nfft,
              int roll, int64_t first_start, int64_t frame_lo, int64_t frame_hi, int64_t k0, int64_t n_out, int dtype,
              void* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Workspace of qi_istft: the windowed inverse transforms of all frames, n_channels * n_frames * nperseg reals, for the
+ * frame lengths one CTA transforms (nfft <= 8192 float32 / 4096 float64); for longer frames those rounded up to 256
+ * bytes plus the pair spectra of up to 65535 frame pairs (multi-pass inverse FFTs). */
+size_t qi_istft_workspace_bytes(int64_t n_channels, int64_t n_frames, int nperseg, int nfft, int dtype);
 
 /* ---- power / information / entropy (tfr_info) -------------------------------------------------
  * `power` is real [M, F, T] (M independent matrices: channels).  All reductions accumulate in fp64. */

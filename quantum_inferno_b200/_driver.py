@@ -154,9 +154,9 @@ def stft(sig, window, nperseg, hop, nfft, n_frames, pad_left, scale, dt, detrend
     nbytes = lib.qi_stft_workspace_bytes(C, int(n_frames), int(nfft), code)
     nbytes = min(nbytes, max(STFT_WORKSPACE_CAP_BYTES, lib.qi_stft_workspace_bytes(C, 2, int(nfft), code)))
     ws = rt.workspace(nbytes) if nbytes else None
-    rc = lib.qi_stft_ws(rt.ptr(sig), C, N, N, rt.ptr(win), int(nperseg), int(hop), int(nfft), int(n_frames),
-                        int(pad_left), float(scale), 1 if detrend else 0, int(roll), code, rt.ptr(out),
-                        rt.ptr(acc), rt.ptr(ws), nbytes, rt.stream())
+    rc = lib.qi_stft(rt.ptr(sig), C, N, N, rt.ptr(win), int(nperseg), int(hop), int(nfft), int(n_frames),
+                     int(pad_left), float(scale), 1 if detrend else 0, int(roll), code, rt.ptr(out),
+                     rt.ptr(acc), rt.ptr(ws), nbytes, rt.stream())
     _lib.check(lib, rc, "qi_stft")
     return acc if psd else out
 
@@ -169,7 +169,7 @@ def istft(spec, dual_win, nperseg, hop, nfft, roll, first_start, frame_lo, frame
     C, P = int(spec.shape[0]), int(spec.shape[2])
     dwin = rt.asarray(np.asarray(dual_win, dtype=np.float64), dt)
     out = rt.empty((C, int(n_out)), dt)
-    nbytes = lib.qi_istft_workspace_bytes_nfft(C, P, int(nperseg), int(nfft), DTYPE_CODE[dt])
+    nbytes = lib.qi_istft_workspace_bytes(C, P, int(nperseg), int(nfft), DTYPE_CODE[dt])
     ws = rt.workspace(nbytes)
     rc = lib.qi_istft(rt.ptr(spec), C, P, rt.ptr(dwin), int(nperseg), int(hop), int(nfft), int(roll), int(first_start),
                       int(frame_lo), int(frame_hi), int(k0), int(n_out), DTYPE_CODE[dt], rt.ptr(out), rt.ptr(ws), nbytes,

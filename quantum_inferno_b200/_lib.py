@@ -14,7 +14,7 @@ QI_F32, QI_F64 = 0, 1
 QI_CONV_LINEAR_SAME, QI_CONV_CIRC_CORR = 0, 1
 QI_CONV_PLAIN_ONLY = 0x100
 SUBSAMPLE_METHOD_CODE = {"nth": 0, "average": 1, "median": 2, "max": 3, "min": 4}
-QI_ABI_VERSION = 4
+QI_ABI_VERSION = 5
 QI_N_CATEGORIES = 7
 CATEGORY_NAMES = ("fft_fwd", "inv_first", "inv_mid", "inv_last", "info", "stft", "other")
 
@@ -58,12 +58,9 @@ SIGNATURES = {
     "qi_stx_multirate_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_vp, _c_int]),
     "qi_stx_multirate": (_c_int, [_c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_int, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "qi_stft": (_c_int, [_c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_dbl, _c_int,
-                         _c_int, _c_int, _c_vp, _c_vp, _c_vp]),
+                         _c_int, _c_int, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "qi_stft_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_int, _c_int]),
-    "qi_stft_ws": (_c_int, [_c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_dbl, _c_int,
-                            _c_int, _c_int, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
-    "qi_istft_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_int, _c_int]),
-    "qi_istft_workspace_bytes_nfft": (_c_sz, [_c_i64, _c_i64, _c_int, _c_int, _c_int]),
+    "qi_istft_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_int, _c_int, _c_int]),
     "qi_istft": (_c_int, [_c_vp, _c_i64, _c_i64, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_i64, _c_i64, _c_i64,
                           _c_i64, _c_int, _c_vp, _c_vp, _c_sz, _c_vp]),
     "qi_power_reduce": (_c_int, [_c_vp, _c_i64, _c_i64, _c_i64, _c_int, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp]),

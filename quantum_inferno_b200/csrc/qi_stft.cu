@@ -14,6 +14,14 @@
 
 namespace qi {
 
+// log2(n) of a power of two n, else -1
+static int log2_pow2(int n) {
+    if (n <= 0 || (n & (n - 1))) return -1;
+    int l = 0;
+    while ((1 << l) < n) ++l;
+    return l;
+}
+
 struct StftGeom {
     i64 n_points, sig_stride, n_frames;
     int nperseg, hop, logF, pad_left, TC, detrend, roll;
@@ -32,6 +40,35 @@ template <typename T> struct StftLaunch {
 // of the Hermitian split (which run along the tiles) on different banks -- one 16-byte element for double; two 8-byte
 // elements for float, which also keeps every tile 16-byte aligned for the vector accesses of the radix-2 stage
 template <typename T> QI_HD int stft_tile_pitch(int R) { return sizeof(T) == 8 ? (pad8(R) | 1) : pad8(R) + 2; }
+
+// Hermitian split of the spectrum Z = Xa + i Xb of two real frames a, b (z1 = Z[k], z2 = Z[nfft - k]) into bin k of both
+// frames, times exp(+2 pi i k roll / nfft): the segment rotated left by roll samples (roll in [0, nfft))
+template <typename T>
+QI_DEV void pair_split(cplx<T> z1, cplx<T> z2, int k, int roll, int logF, cplx<T>& xa, cplx<T>& xb) {
+    const int R = 1 << logF;
+    xa = mk<T>((T)0.5 * (z1.re + z2.re), (T)0.5 * (z1.im - z2.im));
+    xb = mk<T>((T)0.5 * (z1.im + z2.im), (T)-0.5 * (z1.re - z2.re));
+    if (roll) {
+        const cplx<T> ph = unit_root<T>((unsigned long long)(((i64)k * roll) & (R - 1)), logF);
+        xa = xa * ph; xb = xb * ph;
+    }
+}
+
+// Hermitian completion, the inverse of pair_split: bin k <= nfft / 2 of frames a and b, the roll undone, gives
+// zk = Z[k] and zp = Z[nfft - k].  Bins 0 and nfft / 2 are their own partners and lose their imaginary parts, as in
+// irfft: for them the result is false and zp is not to be stored.
+template <typename T>
+QI_DEV bool pair_complete(cplx<T> xa, cplx<T> xb, int k, int roll, int logF, cplx<T>& zk, cplx<T>& zp) {
+    const int R = 1 << logF;
+    if (roll) {
+        const cplx<T> ph = conj(unit_root<T>((unsigned long long)(((i64)k * roll) & (R - 1)), logF));
+        xa = xa * ph; xb = xb * ph;
+    }
+    const bool partner = k != 0 && k != R / 2;
+    zk = partner ? mk<T>(xa.re - xb.im, xa.im + xb.re) : mk<T>(xa.re, xb.re);
+    zp = mk<T>(xa.re + xb.im, xb.re - xa.im);
+    return partner;
+}
 
 // LOGF / LOGTC > 0: FFT length and tiles per CTA known at compile time (the common sizes: every index computation of the
 // gather, the stage loops and the Hermitian split folds to shifts and immediates; ncu of the generic kernel had a third of
@@ -233,12 +270,8 @@ stft_kernel(const T* __restrict__ sig, const T* __restrict__ window, StftGeom g0
         const int k = active ? idx >> logTC : 0;
         const cplx<T> z1 = tile[c * PT + padt<T>((int)brev_bits((unsigned)k, g.logF))];
         const cplx<T> z2 = tile[c * PT + padt<T>((int)brev_bits((unsigned)((R - k) & (R - 1)), g.logF))];
-        cplx<T> xa = mk<T>((T)0.5 * (z1.re + z2.re), (T)0.5 * (z1.im - z2.im));
-        cplx<T> xb = mk<T>((T)0.5 * (z1.im + z2.im), (T)-0.5 * (z1.re - z2.re));
-        if (g.roll) {               // segment rotated left by roll samples: bin k times exp(+2 pi i k roll / nfft)
-            const cplx<T> ph = unit_root<T>((unsigned long long)(((i64)k * g.roll) & (R - 1)), g.logF);
-            xa = xa * ph; xb = xb * ph;
-        }
+        cplx<T> xa, xb;
+        pair_split<T>(z1, z2, k, g.roll, g.logF, xa, xb);
         const i64 fa = frame0 + 2 * c;
         if (out && active) {
             cplx<T>* o = out + (chan * K + k) * g.n_frames + fa;
@@ -269,18 +302,21 @@ template <typename T> static size_t stft_tile_smem(int nfft, int tc) {
 #ifndef QI_STFT_TILE_MAX_NFFT
 #define QI_STFT_TILE_MAX_NFFT 0
 #endif
-// tiles per CTA of stft_kernel, or 0 when one frame does not fit a CTA: <= ~100 KB per CTA so that two CTAs (2 x 512
-// threads) share an SM; one big CTA for long FFTs
-template <typename T> static int stft_tile_columns(int nfft) {
+// tiles per CTA of a tile kernel whose dynamic shared memory is smem(nfft, tiles), or 0 when one frame does not fit a CTA
+// (the long-frame route): down to 2 tiles within `budget` (~100 KB lets two 512-thread CTAs share an SM), then down to
+// one tile in one big CTA of up to 200 KB
+static int tile_columns(int nfft, size_t budget, size_t (*smem)(int nfft, int tc)) {
     if (QI_STFT_TILE_MAX_NFFT > 0 && nfft > QI_STFT_TILE_MAX_NFFT) return 0;
-    size_t budget = StftLaunch<T>::budget;
     int TC = 16;
-    while (TC > 2 && stft_tile_smem<T>(nfft, TC) > budget) TC >>= 1;
-    if (stft_tile_smem<T>(nfft, TC) > budget) {
+    while (TC > 2 && smem(nfft, TC) > budget) TC >>= 1;
+    if (smem(nfft, TC) > budget) {
         budget = 200 * 1024;
-        while (TC > 1 && stft_tile_smem<T>(nfft, TC) > budget) TC >>= 1;
+        while (TC > 1 && smem(nfft, TC) > budget) TC >>= 1;
     }
-    return stft_tile_smem<T>(nfft, TC) > budget ? 0 : TC;
+    return smem(nfft, TC) > budget ? 0 : TC;
+}
+template <typename T> static int stft_tile_columns(int nfft) {
+    return tile_columns(nfft, StftLaunch<T>::budget, stft_tile_smem<T>);
 }
 
 // ---------------------------------------------------------------- frames longer than one CTA's shared memory
@@ -300,6 +336,24 @@ constexpr int STFT_LONG_LOGP = 5, STFT_LONG_P = 1 << STFT_LONG_LOGP;   // positi
 
 // bytes of workspace per frame pair and channel: the pair spectrum and the two frame means
 template <typename T> static size_t stft_long_pair_bytes(int nfft) { return (size_t)nfft * sizeof(cplx<T>) + 2 * sizeof(T); }
+// workspace of the forward: 0 on the tile route, else all frame pairs in one chunk
+template <typename T> static size_t stft_workspace_bytes(i64 C, i64 n_frames, int nfft) {
+    if (stft_tile_columns<T>(nfft)) return 0;
+    return (size_t)C * (size_t)((n_frames + 1) / 2) * stft_long_pair_bytes<T>(nfft);
+}
+
+// frame pairs per channel in one chunk: all of them, but at most 65535 / C (the C npc batch rows of a launch are grid.y)
+static i64 long_pairs_per_chunk(i64 C, i64 n_frames) {
+    const i64 npairs = (n_frames + 1) / 2, cap = 65535 / C;
+    return npairs < cap ? npairs : cap;
+}
+
+// batch row b of a chunk (npc pairs per channel from pair p0 on): its channel and its first frame
+struct PairRow { i64 chan, fa; };
+QI_DEV PairRow pair_row(i64 b, int npc, i64 p0) {
+    const unsigned bu = (unsigned)b;                      // b < 65536 (grid.y)
+    return {(i64)(bu / (unsigned)npc), 2 * (p0 + bu % (unsigned)npc)};
+}
 
 // mean of frame f0 + blockIdx.x over its nperseg samples of the zero-extended record, summed in fp64 and rounded to T as
 // stft_kernel does; frames >= n_frames get 0.  means[chan][gridDim.x]
@@ -330,12 +384,11 @@ template <typename T> struct SrcStftPair {
     int npc, nperseg, hop, pad_left;
     QI_DEV cplx<T> load(i64 b, i64 e) const {
         if (e >= nperseg) return mk<T>((T)0, (T)0);
-        const unsigned bu = (unsigned)b;                  // b < 65536 (grid.y)
-        const i64 chan = bu / (unsigned)npc, fa = 2 * (p0 + bu % (unsigned)npc);
-        const T* x = sig + chan * sig_stride;
-        const i64 pa = fa * hop + e - pad_left, pb = pa + hop;
-        T va = fa < n_frames && pa >= 0 && pa < n_points ? x[pa] : (T)0;
-        T vb = fa + 1 < n_frames && pb >= 0 && pb < n_points ? x[pb] : (T)0;
+        const PairRow r = pair_row(b, npc, p0);
+        const T* x = sig + r.chan * sig_stride;
+        const i64 pa = r.fa * hop + e - pad_left, pb = pa + hop;
+        T va = r.fa < n_frames && pa >= 0 && pa < n_points ? x[pa] : (T)0;
+        T vb = r.fa + 1 < n_frames && pb >= 0 && pb < n_points ? x[pb] : (T)0;
         if (means) { va -= means[2 * b]; vb -= means[2 * b + 1]; }
         const T w = window[e];
         return mk<T>(va * w, vb * w);
@@ -345,9 +398,39 @@ template <typename T> struct SrcStftPair {
 // shared-memory slot of storage offset i of block q (0: residue c, 1: its partner) for frame pair t
 QI_HD int stft_long_slot(int q, int t, int i) { return (q * STFT_LONG_P + t) * (STFT_LONG_P + 1) + i; }
 
+// The block pair of one CTA of stft_split_kernel / istft_gather_kernel, grid = (nblk / 2 + 1, ceil(npc / P), C) with
+// nblk = nfft / P: blocks c = blockIdx.x and c2 = nblk - c (nb = 1 when they coincide), frame pairs t0 .. t0 + ntp - 1
+// of the chunk.  Slot q P + j of the pair is bin k = (q ? c2 : c) + j nfft / P at position i of its block; its Hermitian
+// partner k2 = nfft - k sits at position i2 of block q2.
+struct LongBlockPair {
+    int logL, nblk, c, c2, nb, t0, ntp;
+    struct Slot { int q, k, i, k2, q2, i2; };
+    QI_DEV LongBlockPair(int logL_, int npc)
+        : logL(logL_), nblk((1 << logL_) >> STFT_LONG_LOGP), c(blockIdx.x), c2((nblk - c) & (nblk - 1)),
+          nb(c2 == c ? 1 : 2), t0(blockIdx.y * STFT_LONG_P), ntp(npc - t0 < STFT_LONG_P ? npc - t0 : STFT_LONG_P) {}
+    // storage position of element 0 of block q in a bit-reversed row
+    QI_DEV unsigned row_pos(int q) const { return brev_bits((unsigned)(q ? c2 : c), logL); }
+    QI_DEV Slot slot(int s) const {
+        constexpr int logP = STFT_LONG_LOGP;
+        const int q = s >> logP, j = s & (STFT_LONG_P - 1);
+        const int k = (q ? c2 : c) + (j << (logL - logP));
+        const int k2 = ((1 << logL) - k) & ((1 << logL) - 1);
+        return {q, k, (int)brev_bits((unsigned)j, logP), k2, (k2 & (nblk - 1)) == c ? 0 : 1,
+                (int)brev_bits((unsigned)(k2 >> (logL - logP)), logP)};
+    }
+};
+// launch geometry of those kernels for a chunk of npc frame pairs per channel: 256 threads and this grid and shared memory
+static dim3 long_pair_grid(int logL, int npc, i64 C) {
+    return dim3((unsigned)(((1 << logL) >> STFT_LONG_LOGP) / 2 + 1), (unsigned)((npc + STFT_LONG_P - 1) / STFT_LONG_P),
+                (unsigned)C);
+}
+template <typename T> static size_t long_pair_smem() {
+    return (size_t)2 * STFT_LONG_P * (STFT_LONG_P + 1) * sizeof(cplx<T>);
+}
+
 // Hermitian split of the pair spectra of one chunk (buf [C * npc][nfft], bit-reversed) into the one-sided bins of both
 // frames, times the roll phase and the scale: out [C, nfft/2+1, n_frames] and / or psd_acc [C, nfft/2+1] += |X_k|^2.
-// grid = (nfft / (2 LP) + 1 block pairs, ceil(npc / LP), C); 256 threads; one warp per bin, lanes along the frame pairs.
+// 256 threads; one warp per bin, lanes along the frame pairs.
 template <typename T>
 __global__ void __launch_bounds__(256)
 stft_split_kernel(const cplx<T>* __restrict__ buf, int logL, int npc, i64 p0, i64 n_frames, int roll, T sc,
@@ -355,44 +438,37 @@ stft_split_kernel(const cplx<T>* __restrict__ buf, int logL, int npc, i64 p0, i6
     QI_DYN_SMEM(smem_raw);
     constexpr int P = STFT_LONG_P, logP = STFT_LONG_LOGP;
     cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
-    const int L = 1 << logL, nblk = L >> logP, K = (L >> 1) + 1;
-    const int c = blockIdx.x, c2 = (nblk - c) & (nblk - 1), nb = c2 == c ? 1 : 2;
-    const int t0 = blockIdx.y * P, ntp = npc - t0 < P ? npc - t0 : P;
+    const int L = 1 << logL, K = (L >> 1) + 1;
+    const LongBlockPair bp(logL, npc);
     const i64 chan = blockIdx.z;
-    const cplx<T>* rows = buf + (chan * npc + t0) * (i64)L;
-    for (int idx = threadIdx.x; idx < nb * P * P; idx += blockDim.x) {     // lanes along the positions of one row
+    const cplx<T>* rows = buf + (chan * npc + bp.t0) * (i64)L;
+    for (int idx = threadIdx.x; idx < bp.nb * P * P; idx += blockDim.x) {  // lanes along the positions of one row
         const int i = idx & (P - 1), t = (idx >> logP) & (P - 1), q = idx >> (2 * logP);
-        if (t < ntp) s[stft_long_slot(q, t, i)] = rows[(i64)t * L + brev_bits((unsigned)(q ? c2 : c), logL) + i];
+        if (t < bp.ntp) s[stft_long_slot(q, t, i)] = rows[(i64)t * L + bp.row_pos(q) + i];
     }
     __syncthreads();
     const int t = threadIdx.x & 31;
-    const i64 fa = 2 * (p0 + t0 + t);
-    for (int slot = threadIdx.x >> 5; slot < nb * P; slot += blockDim.x >> 5) {
-        const int q = slot >> logP, j = slot & (P - 1);
-        const int k = (q ? c2 : c) + (j << (logL - logP));
+    const i64 fa = 2 * (p0 + bp.t0 + t);
+    for (int slot = threadIdx.x >> 5; slot < bp.nb * P; slot += blockDim.x >> 5) {
+        const LongBlockPair::Slot sl = bp.slot(slot);
+        const int k = sl.k;
         if (k > (L >> 1)) continue;                                       // the partner's warp has it
-        const int k2 = (L - k) & (L - 1);
-        const int q2 = (k2 & (nblk - 1)) == c ? 0 : 1;
         cplx<T> z1 = mk<T>((T)0, (T)0), z2 = z1;
-        if (t < ntp) {
-            z1 = s[stft_long_slot(q, t, (int)brev_bits((unsigned)j, logP))];
-            z2 = s[stft_long_slot(q2, t, (int)brev_bits((unsigned)(k2 >> (logL - logP)), logP))];
+        if (t < bp.ntp) {
+            z1 = s[stft_long_slot(sl.q, t, sl.i)];
+            z2 = s[stft_long_slot(sl.q2, t, sl.i2)];
         }
-        cplx<T> xa = mk<T>((T)0.5 * (z1.re + z2.re), (T)0.5 * (z1.im - z2.im));
-        cplx<T> xb = mk<T>((T)0.5 * (z1.im + z2.im), (T)-0.5 * (z1.re - z2.re));
-        if (roll) {
-            const cplx<T> ph = unit_root<T>((unsigned long long)(((i64)k * roll) & (L - 1)), logL);
-            xa = xa * ph; xb = xb * ph;
-        }
-        if (out && t < ntp) {
+        cplx<T> xa, xb;
+        pair_split<T>(z1, z2, k, roll, logL, xa, xb);
+        if (out && t < bp.ntp) {
             cplx<T>* o = out + (chan * K + k) * n_frames + fa;
             if (fa < n_frames) o[0] = xa * sc;
             if (fa + 1 < n_frames) o[1] = xb * sc;
         }
         if (psd_acc) {
             double pw = 0.0;
-            if (t < ntp && fa < n_frames) pw += (double)norm2(xa);
-            if (t < ntp && fa + 1 < n_frames) pw += (double)norm2(xb);
+            if (t < bp.ntp && fa < n_frames) pw += (double)norm2(xa);
+            if (t < bp.ntp && fa + 1 < n_frames) pw += (double)norm2(xb);
             pw = warp_sum(pw);
             if (t == 0) atomicAdd(&psd_acc[chan * K + k], pw);
         }
@@ -408,14 +484,11 @@ static int stft_long(const T* sig, i64 C, i64 n_points, i64 stride, const T* win
     if (ws_bytes < per_pair) return QI_ERR_WORKSPACE;
     if (reinterpret_cast<uintptr_t>(ws) % sizeof(cplx<T>)) return QI_ERR_ARG;
     const i64 npairs = (n_frames + 1) / 2;
-    i64 npc = (i64)(ws_bytes / per_pair);
-    if (npc > 65535 / C) npc = 65535 / C;                 // batch rows per launch: grid.y
-    if (npc > npairs) npc = npairs;
+    i64 npc = long_pairs_per_chunk(C, n_frames);
+    if (npc > (i64)(ws_bytes / per_pair)) npc = (i64)(ws_bytes / per_pair);
     cplx<T>* buf = static_cast<cplx<T>*>(ws);
     T* means = reinterpret_cast<T*>(buf + (size_t)C * npc * L);
     const FftPlan plan = make_plan(logL, (int)sizeof(cplx<T>));
-    const int nblk = L >> STFT_LONG_LOGP;
-    const size_t split_smem = (size_t)2 * STFT_LONG_P * (STFT_LONG_P + 1) * sizeof(cplx<T>);
     if (psd_acc) cudaMemsetAsync(psd_acc, 0, sizeof(double) * (size_t)C * (L / 2 + 1), st);
     for (i64 p0 = 0; p0 < npairs; p0 += npc) {
         const int n = (int)(npairs - p0 < npc ? npairs - p0 : npc);
@@ -426,31 +499,30 @@ static int stft_long(const T* sig, i64 C, i64 n_points, i64 stride, const T* win
         const SrcStftPair<T> src{sig, window, detrend ? means : nullptr, stride, n_points, n_frames, p0, n, nperseg, hop,
                                  pad_left};
         forward_passes<T>(plan, C * n, src, buf, L, st);
-        QI_LAUNCH((stft_split_kernel<T>), dim3((unsigned)(nblk / 2 + 1), (unsigned)((n + STFT_LONG_P - 1) / STFT_LONG_P),
-                  (unsigned)C), dim3(256), split_smem, st, buf, logL, n, p0, n_frames, roll, (T)scale, out, psd_acc);
+        QI_LAUNCH((stft_split_kernel<T>), long_pair_grid(logL, n, C), dim3(256), long_pair_smem<T>(), st, buf, logL, n, p0,
+                  n_frames, roll, (T)scale, out, psd_acc);
     }
     return check_cuda("qi_stft");
 }
 
+// nfft = 2^logF; roll in [0, nfft)
 template <typename T>
 static int stft_impl(const void* sig, i64 C, i64 n_points, i64 stride, const void* window, int nperseg, int hop,
-                     int nfft, i64 n_frames, int pad_left, double scale, int detrend, int roll, void* out,
+                     int logF, i64 n_frames, int pad_left, double scale, int detrend, int roll, void* out,
                      double* psd_acc, void* ws, size_t ws_bytes, cudaStream_t st) {
-    int logF = 0;
-    while ((1 << logF) < nfft) ++logF;
-    if ((1 << logF) != nfft) return QI_ERR_ARG;
+    const int nfft = 1 << logF;
     const int TC = stft_tile_columns<T>(nfft);
     if (TC == 0 && !ws) return QI_ERR_UNSUPPORTED;
     if (C > 65535) return QI_ERR_UNSUPPORTED;
     if (TC == 0)
         return stft_long<T>(static_cast<const T*>(sig), C, n_points, stride, static_cast<const T*>(window), nperseg, hop,
-                            logF, n_frames, pad_left, scale, detrend, ((roll % nfft) + nfft) % nfft,
-                            static_cast<cplx<T>*>(out), psd_acc, ws, ws_bytes, st);
+                            logF, n_frames, pad_left, scale, detrend, roll, static_cast<cplx<T>*>(out), psd_acc, ws,
+                            ws_bytes, st);
     // the psd reduction uses shuffles across the TC lanes of one k: needs TC | 32 (true: power of two <= 16)
     StftGeom g;
     g.n_points = n_points; g.sig_stride = stride; g.n_frames = n_frames;
     g.nperseg = nperseg; g.hop = hop; g.logF = logF; g.pad_left = pad_left; g.TC = TC; g.detrend = detrend;
-    g.roll = ((roll % nfft) + nfft) % nfft;
+    g.roll = roll;
     g.scale = scale;
     dim3 grid((unsigned)((n_frames + 2 * TC - 1) / (2 * TC)), (unsigned)C);
     const size_t smem = stft_tile_smem<T>(nfft, TC);
@@ -526,17 +598,10 @@ istft_frames_kernel(const cplx<T>* __restrict__ S, const T* __restrict__ dual_wi
             if (idx >= K * TC) continue;
             const int c = idx & (TC - 1);
             const int k = idx >> logTC;
-            cplx<T> xa = xa_[u], xb = xb_[u];
-            if (g.roll) {           // undo the rotation of the forward transform: bin k times exp(-2 pi i k roll / nfft)
-                const cplx<T> ph = conj(unit_root<T>((unsigned long long)(((i64)k * g.roll) & (R - 1)), g.logF));
-                xa = xa * ph; xb = xb * ph;
-            }
-            if (k == 0 || k == R / 2) {                                    // irfft ignores these imaginary parts
-                tile[(int)brev_bits((unsigned)k, g.logF) * TP + c] = mk<T>(xa.re, xb.re);
-            } else {
-                tile[(int)brev_bits((unsigned)k, g.logF) * TP + c] = mk<T>(xa.re - xb.im, xa.im + xb.re);
-                tile[(int)brev_bits((unsigned)(R - k), g.logF) * TP + c] = mk<T>(xa.re + xb.im, xb.re - xa.im);
-            }
+            cplx<T> zk, zp;
+            const bool partner = pair_complete<T>(xa_[u], xb_[u], k, g.roll, g.logF, zk, zp);
+            tile[(int)brev_bits((unsigned)k, g.logF) * TP + c] = zk;
+            if (partner) tile[(int)brev_bits((unsigned)(R - k), g.logF) * TP + c] = zp;
         }
     }
     __syncthreads();
@@ -582,21 +647,11 @@ istft_ola_kernel(const T* __restrict__ slices, IstftGeom g, T* __restrict__ out)
 }
 
 // dynamic shared memory of istft_frames_kernel with tc columns, and its columns per CTA (0: the frame does not fit)
-static size_t istft_tile_smem(int nfft, int tc, size_t elem_bytes) { return (size_t)nfft * (tc + 2) * elem_bytes + 64; }
-template <typename T> static int istft_tile_columns(int nfft) {
-    size_t budget = 100 * 1024;
-    int TC = 16;
-    while (TC > 2 && istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) TC >>= 1;
-    if (istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) {
-        budget = 200 * 1024;
-        while (TC > 1 && istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget) TC >>= 1;
-    }
-    return istft_tile_smem(nfft, TC, sizeof(cplx<T>)) > budget ? 0 : TC;
-}
+template <typename T> static size_t istft_tile_smem(int nfft, int tc) { return (size_t)nfft * (tc + 2) * sizeof(cplx<T>) + 64; }
+template <typename T> static int istft_tile_columns(int nfft) { return tile_columns(nfft, 100 * 1024, istft_tile_smem<T>); }
 
 // Long frames: Hermitian-completed pair spectra Z = Xa + i Xb of one chunk (S [C, nfft/2+1, P] -> buf [C * npc][nfft],
-// bit-reversed rows), the roll undone; the imaginary parts of bins 0 and nfft/2 dropped as irfft does.  Same grid and
-// block pairing as stft_split_kernel.
+// bit-reversed rows).  The block pairs of stft_split_kernel, the other way round.
 template <typename T>
 __global__ void __launch_bounds__(256)
 istft_gather_kernel(const cplx<T>* __restrict__ S, int logL, int npc, i64 p0, i64 n_frames, int roll,
@@ -604,38 +659,28 @@ istft_gather_kernel(const cplx<T>* __restrict__ S, int logL, int npc, i64 p0, i6
     QI_DYN_SMEM(smem_raw);
     constexpr int P = STFT_LONG_P, logP = STFT_LONG_LOGP;
     cplx<T>* s = reinterpret_cast<cplx<T>*>(smem_raw);
-    const int L = 1 << logL, nblk = L >> logP, K = (L >> 1) + 1;
-    const int c = blockIdx.x, c2 = (nblk - c) & (nblk - 1), nb = c2 == c ? 1 : 2;
-    const int t0 = blockIdx.y * P, ntp = npc - t0 < P ? npc - t0 : P;
+    const int L = 1 << logL, K = (L >> 1) + 1;
+    const LongBlockPair bp(logL, npc);
     const i64 chan = blockIdx.z;
     const int t = threadIdx.x & 31;
-    const i64 fa = 2 * (p0 + t0 + t);
-    for (int slot = threadIdx.x >> 5; slot < nb * P; slot += blockDim.x >> 5) {
-        const int q = slot >> logP, j = slot & (P - 1);
-        const int k = (q ? c2 : c) + (j << (logL - logP));
-        if (k > (L >> 1) || t >= ntp) continue;                          // bins above nfft/2: the partner's warp
-        const int k2 = (L - k) & (L - 1);
-        const int q2 = (k2 & (nblk - 1)) == c ? 0 : 1;
+    const i64 fa = 2 * (p0 + bp.t0 + t);
+    for (int slot = threadIdx.x >> 5; slot < bp.nb * P; slot += blockDim.x >> 5) {
+        const LongBlockPair::Slot sl = bp.slot(slot);
+        const int k = sl.k;
+        if (k > (L >> 1) || t >= bp.ntp) continue;                       // bins above nfft/2: the partner's warp
         cplx<T> xa = mk<T>((T)0, (T)0), xb = xa;
         if (fa < n_frames) xa = S[(chan * K + k) * n_frames + fa];
         if (fa + 1 < n_frames) xb = S[(chan * K + k) * n_frames + fa + 1];
-        if (roll) {
-            const cplx<T> ph = conj(unit_root<T>((unsigned long long)(((i64)k * roll) & (L - 1)), logL));
-            xa = xa * ph; xb = xb * ph;
-        }
-        const int i1 = (int)brev_bits((unsigned)j, logP);
-        if (k == 0 || k == (L >> 1)) {
-            s[stft_long_slot(q, t, i1)] = mk<T>(xa.re, xb.re);
-        } else {
-            s[stft_long_slot(q, t, i1)] = mk<T>(xa.re - xb.im, xa.im + xb.re);
-            s[stft_long_slot(q2, t, (int)brev_bits((unsigned)(k2 >> (logL - logP)), logP))] = mk<T>(xa.re + xb.im, xb.re - xa.im);
-        }
+        cplx<T> zk, zp;
+        const bool partner = pair_complete<T>(xa, xb, k, roll, logL, zk, zp);
+        s[stft_long_slot(sl.q, t, sl.i)] = zk;
+        if (partner) s[stft_long_slot(sl.q2, t, sl.i2)] = zp;
     }
     __syncthreads();
-    cplx<T>* rows = buf + (chan * npc + t0) * (i64)L;
-    for (int idx = threadIdx.x; idx < nb * P * P; idx += blockDim.x) {     // lanes along the positions of one row
+    cplx<T>* rows = buf + (chan * npc + bp.t0) * (i64)L;
+    for (int idx = threadIdx.x; idx < bp.nb * P * P; idx += blockDim.x) {  // lanes along the positions of one row
         const int i = idx & (P - 1), tt = (idx >> logP) & (P - 1), q = idx >> (2 * logP);
-        if (tt < ntp) rows[(i64)tt * L + brev_bits((unsigned)(q ? c2 : c), logL) + i] = s[stft_long_slot(q, tt, i)];
+        if (tt < bp.ntp) rows[(i64)tt * L + bp.row_pos(q) + i] = s[stft_long_slot(q, tt, i)];
     }
 }
 
@@ -648,65 +693,62 @@ template <typename T> struct DstIstftPair {
     T inv;
     QI_DEV void store(i64 b, i64 n, cplx<T> v) const {
         if (n >= nperseg) return;
-        const unsigned bu = (unsigned)b;                  // b < 65536 (grid.y)
-        const i64 chan = bu / (unsigned)npc, fa = 2 * (p0 + bu % (unsigned)npc);
+        const PairRow r = pair_row(b, npc, p0);
         const T w = dual_win[n] * inv;
-        T* o = slices + (chan * n_frames + fa) * nperseg + n;
+        T* o = slices + (r.chan * n_frames + r.fa) * nperseg + n;
         o[0] = v.re * w;
-        if (fa + 1 < n_frames) o[nperseg] = v.im * w;
+        if (r.fa + 1 < n_frames) o[nperseg] = v.im * w;
     }
     QI_DEV void finish(i64, unsigned char*) const {}
 };
 
-// long-route workspace: the slices (rounded up to 256 bytes), then the pair spectra of one chunk
-static i64 istft_long_pairs_per_chunk(i64 C, i64 n_frames) {
-    const i64 npairs = (n_frames + 1) / 2, cap = 65535 / C;
-    return npairs < cap ? npairs : cap;
+// workspace of the inverse: the slices; on the long route those rounded up to 256 bytes, then the pair spectra of one chunk
+template <typename T> static size_t istft_slices_bytes(i64 C, i64 n_frames, int nperseg) {
+    return (size_t)C * (size_t)n_frames * (size_t)nperseg * sizeof(T);
 }
-static size_t istft_slices_bytes(i64 C, i64 n_frames, int nperseg, size_t real_bytes) {
-    return (size_t)C * (size_t)n_frames * (size_t)nperseg * real_bytes;
+template <typename T> static size_t istft_workspace_bytes(i64 C, i64 n_frames, int nperseg, int nfft) {
+    const size_t slices = istft_slices_bytes<T>(C, n_frames, nperseg);
+    if (C > 65535 || log2_pow2(nfft) < 0 || istft_tile_columns<T>(nfft)) return slices;
+    return (slices + 255) / 256 * 256 + (size_t)C * (size_t)long_pairs_per_chunk(C, n_frames) * (size_t)nfft * sizeof(cplx<T>);
 }
 
 template <typename T>
 static void istft_long_slices(const cplx<T>* S, i64 C, i64 P, const T* dual_win, int nperseg, int logL, int roll, T* slices,
                               cudaStream_t st) {
     const int L = 1 << logL;
-    const i64 npairs = (P + 1) / 2, npc = istft_long_pairs_per_chunk(C, P);
+    const i64 npairs = (P + 1) / 2, npc = long_pairs_per_chunk(C, P);
     cplx<T>* buf = reinterpret_cast<cplx<T>*>(reinterpret_cast<unsigned char*>(slices) +
-                                              (istft_slices_bytes(C, P, nperseg, sizeof(T)) + 255) / 256 * 256);
+                                              (istft_slices_bytes<T>(C, P, nperseg) + 255) / 256 * 256);
     const FftPlan plan = make_plan(logL, (int)sizeof(cplx<T>));
-    const int nblk = L >> STFT_LONG_LOGP;
-    const size_t smem = (size_t)2 * STFT_LONG_P * (STFT_LONG_P + 1) * sizeof(cplx<T>);
     const T inv = (T)(1.0 / (double)L);
     for (i64 p0 = 0; p0 < npairs; p0 += npc) {
         const int n = (int)(npairs - p0 < npc ? npairs - p0 : npc);
         prof_set_category(QI_CAT_STFT);
-        QI_LAUNCH((istft_gather_kernel<T>), dim3((unsigned)(nblk / 2 + 1), (unsigned)((n + STFT_LONG_P - 1) / STFT_LONG_P),
-                  (unsigned)C), dim3(256), smem, st, S, logL, n, p0, P, roll, buf);
+        QI_LAUNCH((istft_gather_kernel<T>), long_pair_grid(logL, n, C), dim3(256), long_pair_smem<T>(), st, S, logL, n, p0,
+                  P, roll, buf);
         const DstIstftPair<T> dst{slices, dual_win, P, p0, n, nperseg, inv};
         inverse_passes<T>(plan, C * n, SrcComplex<T>{buf, L}, dst, 0, false, buf, L, st);
     }
     prof_set_category(QI_CAT_STFT);
 }
 
+// nfft = 2^logF; roll in [0, nfft)
 template <typename T>
-static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int nperseg, int hop, int nfft, int roll,
+static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int nperseg, int hop, int logF, int roll,
                       i64 first_start, i64 frame_lo, i64 frame_hi, i64 k0, i64 n_out, void* out, void* ws,
                       cudaStream_t st) {
-    int logF = 0;
-    while ((1 << logF) < nfft) ++logF;
-    if ((1 << logF) != nfft) return QI_ERR_ARG;
+    const int nfft = 1 << logF;
     const int TC = istft_tile_columns<T>(nfft);
     if (C > 65535) return QI_ERR_UNSUPPORTED;
     IstftGeom g;
     g.n_frames = P; g.first_start = first_start; g.frame_lo = frame_lo; g.frame_hi = frame_hi; g.k0 = k0; g.n_out = n_out;
-    g.nperseg = nperseg; g.hop = hop; g.logF = logF; g.TC = TC; g.roll = ((roll % nfft) + nfft) % nfft;
+    g.nperseg = nperseg; g.hop = hop; g.logF = logF; g.TC = TC; g.roll = roll;
     if (TC == 0) {
         if (reinterpret_cast<uintptr_t>(ws) % sizeof(cplx<T>)) return QI_ERR_ARG;
-        istft_long_slices<T>(static_cast<const cplx<T>*>(S), C, P, static_cast<const T*>(dual_win), nperseg, logF, g.roll,
+        istft_long_slices<T>(static_cast<const cplx<T>*>(S), C, P, static_cast<const T*>(dual_win), nperseg, logF, roll,
                              static_cast<T*>(ws), st);
     } else {
-        const size_t smem = istft_tile_smem(nfft, TC, sizeof(cplx<T>));
+        const size_t smem = istft_tile_smem<T>(nfft, TC);
 #ifndef QI_EMUL
         cudaFuncSetAttribute(istft_frames_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 #endif
@@ -722,32 +764,37 @@ static int istft_impl(const void* S, i64 C, i64 P, const void* dual_win, int npe
 
 }  // namespace qi
 
-namespace {
-bool is_pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }
-// true when the tile kernels refuse this frame length in this dtype (the long-frame route takes it)
-bool long_frames(int nfft, int dtype, bool inverse) {
-    if (!is_pow2(nfft) || (dtype != QI_F32 && dtype != QI_F64)) return false;
-    if (inverse) return (dtype == QI_F64 ? qi::istft_tile_columns<double>(nfft) : qi::istft_tile_columns<float>(nfft)) == 0;
-    return (dtype == QI_F64 ? qi::stft_tile_columns<double>(nfft) : qi::stft_tile_columns<float>(nfft)) == 0;
-}
-}  // namespace
-
 extern "C" size_t qi_stft_workspace_bytes(int64_t C, int64_t n_frames, int nfft, int dtype) {
-    if (C <= 0 || n_frames <= 0 || !long_frames(nfft, dtype, false)) return 0;
-    const size_t per_pair = dtype == QI_F64 ? qi::stft_long_pair_bytes<double>(nfft) : qi::stft_long_pair_bytes<float>(nfft);
-    return (size_t)C * (size_t)((n_frames + 1) / 2) * per_pair;
+    if (C <= 0 || n_frames <= 0 || qi::log2_pow2(nfft) < 0) return 0;
+    if (dtype == QI_F32) return qi::stft_workspace_bytes<float>(C, n_frames, nfft);
+    if (dtype == QI_F64) return qi::stft_workspace_bytes<double>(C, n_frames, nfft);
+    return 0;
 }
 
-extern "C" size_t qi_istft_workspace_bytes(int64_t C, int64_t n_frames, int nperseg, int dtype) {
+extern "C" int qi_stft(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window, int nperseg,
+                       int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll, int dtype,
+                       void* out, double* psd_acc, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!sig || !window || C <= 0 || n_points <= 0 || nperseg <= 0 || hop <= 0 || nfft < nperseg || n_frames <= 0)
+        return QI_ERR_ARG;
+    if (!out && !psd_acc) return QI_ERR_ARG;
+    const int logF = qi::log2_pow2(nfft);
+    if (logF < 0) return QI_ERR_ARG;
+    roll = ((roll % nfft) + nfft) % nfft;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (dtype == QI_F32)
+        return qi::stft_impl<float>(sig, C, n_points, stride, window, nperseg, hop, logF, n_frames, pad_left, scale,
+                                    detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
+    if (dtype == QI_F64)
+        return qi::stft_impl<double>(sig, C, n_points, stride, window, nperseg, hop, logF, n_frames, pad_left, scale,
+                                     detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
+    return QI_ERR_ARG;
+}
+
+extern "C" size_t qi_istft_workspace_bytes(int64_t C, int64_t n_frames, int nperseg, int nfft, int dtype) {
     if (C <= 0 || n_frames <= 0 || nperseg <= 0) return 0;
-    return qi::istft_slices_bytes(C, n_frames, nperseg, dtype == QI_F64 ? 8 : 4);
-}
-
-extern "C" size_t qi_istft_workspace_bytes_nfft(int64_t C, int64_t n_frames, int nperseg, int nfft, int dtype) {
-    const size_t slices = qi_istft_workspace_bytes(C, n_frames, nperseg, dtype);
-    if (slices == 0 || C > 65535 || !long_frames(nfft, dtype, true)) return slices;
-    return (slices + 255) / 256 * 256 +
-           (size_t)C * (size_t)qi::istft_long_pairs_per_chunk(C, n_frames) * (size_t)nfft * (dtype == QI_F64 ? 16 : 8);
+    if (dtype == QI_F64) return qi::istft_workspace_bytes<double>(C, n_frames, nperseg, nfft);
+    // float32; for an unknown dtype, which qi_istft refuses, the float32 slices alone
+    return qi::istft_workspace_bytes<float>(C, n_frames, nperseg, dtype == QI_F32 ? nfft : 0);
 }
 
 extern "C" int qi_istft(const void* S, int64_t C, int64_t n_frames, const void* dual_win, int nperseg, int hop, int nfft,
@@ -756,37 +803,16 @@ extern "C" int qi_istft(const void* S, int64_t C, int64_t n_frames, const void* 
     if (!S || !dual_win || !out || !ws || C <= 0 || n_frames <= 0 || nperseg <= 0 || hop <= 0 || nfft < nperseg ||
         n_out <= 0 || frame_lo < 0 || frame_hi > n_frames || frame_lo >= frame_hi)
         return QI_ERR_ARG;
-    if (ws_bytes < qi_istft_workspace_bytes_nfft(C, n_frames, nperseg, nfft, dtype)) return QI_ERR_WORKSPACE;
+    if (ws_bytes < qi_istft_workspace_bytes(C, n_frames, nperseg, nfft, dtype)) return QI_ERR_WORKSPACE;
+    const int logF = qi::log2_pow2(nfft);
+    if (logF < 0) return QI_ERR_ARG;
+    roll = ((roll % nfft) + nfft) % nfft;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (dtype == QI_F32)
-        return qi::istft_impl<float>(S, C, n_frames, dual_win, nperseg, hop, nfft, roll, first_start, frame_lo, frame_hi,
+        return qi::istft_impl<float>(S, C, n_frames, dual_win, nperseg, hop, logF, roll, first_start, frame_lo, frame_hi,
                                      k0, n_out, out, ws, st);
     if (dtype == QI_F64)
-        return qi::istft_impl<double>(S, C, n_frames, dual_win, nperseg, hop, nfft, roll, first_start, frame_lo,
+        return qi::istft_impl<double>(S, C, n_frames, dual_win, nperseg, hop, logF, roll, first_start, frame_lo,
                                       frame_hi, k0, n_out, out, ws, st);
     return QI_ERR_ARG;
-}
-
-extern "C" int qi_stft_ws(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window,
-                          int nperseg, int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend,
-                          int roll, int dtype, void* out, double* psd_acc, void* workspace, size_t workspace_bytes,
-                          void* stream) {
-    if (!sig || !window || C <= 0 || n_points <= 0 || nperseg <= 0 || hop <= 0 || nfft < nperseg || n_frames <= 0)
-        return QI_ERR_ARG;
-    if (!out && !psd_acc) return QI_ERR_ARG;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (dtype == QI_F32)
-        return qi::stft_impl<float>(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale,
-                                    detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
-    if (dtype == QI_F64)
-        return qi::stft_impl<double>(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale,
-                                     detrend, roll, out, psd_acc, workspace, workspace_bytes, st);
-    return QI_ERR_ARG;
-}
-
-extern "C" int qi_stft(const void* sig, int64_t C, int64_t n_points, int64_t stride, const void* window, int nperseg,
-                       int hop, int nfft, int64_t n_frames, int pad_left, double scale, int detrend, int roll, int dtype,
-                       void* out, double* psd_acc, void* stream) {
-    return qi_stft_ws(sig, C, n_points, stride, window, nperseg, hop, nfft, n_frames, pad_left, scale, detrend, roll,
-                      dtype, out, psd_acc, nullptr, 0, stream);
 }

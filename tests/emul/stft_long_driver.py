@@ -34,8 +34,8 @@ with _runtime.use_runtime(EmulRuntime()) as rt:
     ws = rt.workspace(ws_min)
     out = rt.empty((2, 8193, n_frames), "complex128")
     acc = rt.empty((2, 8193), "float64")
-    rc = lib.qi_stft_ws(rt.ptr(x), 2, 30000, 30000, rt.ptr(win), 16384, 6000, 16384, n_frames, 8192, 1.0, 1, 5, code,
-                        rt.ptr(out), rt.ptr(acc), rt.ptr(ws), ws_min, None)
+    rc = lib.qi_stft(rt.ptr(x), 2, 30000, 30000, rt.ptr(win), 16384, 6000, 16384, n_frames, 8192, 1.0, 1, 5, code,
+                     rt.ptr(out), rt.ptr(acc), rt.ptr(ws), ws_min, None)
     print("minimum workspace", rc, flush=True)
     assert rc == 0
 print("asan run done")

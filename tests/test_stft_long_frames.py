@@ -121,22 +121,23 @@ def _c_stft(rt, x, nperseg, hop, nfft, n_frames, pad_left, dt, ws_bytes, roll=0,
     out = None if psd else rt.zeros((C, nfft // 2 + 1, n_frames), "complex128" if dt == "float64" else "complex64")
     acc = rt.zeros((C, nfft // 2 + 1), "float64") if psd else None
     buf = rt.workspace(ws_bytes) if ws else None
-    rc = lib.qi_stft_ws(rt.ptr(xs), C, N, N, rt.ptr(win), nperseg, hop, nfft, n_frames, pad_left, 0.5, 1, roll, code,
-                        rt.ptr(out), rt.ptr(acc), rt.ptr(buf), ws_bytes, None)
+    rc = lib.qi_stft(rt.ptr(xs), C, N, N, rt.ptr(win), nperseg, hop, nfft, n_frames, pad_left, 0.5, 1, roll, code,
+                     rt.ptr(out), rt.ptr(acc), rt.ptr(buf), ws_bytes, None)
     return rc, (acc if psd else out)
 
 
-def test_c_abi_workspace_and_chunking(emul):
+def test_c_abi_one_entry_per_direction_workspace_and_chunking(emul):
+    """qi_stft with and without a workspace, and the workspace sizes of both directions"""
     from quantum_inferno_b200 import _lib
     lib = emul.lib
-    # every size the one-CTA kernels take needs no workspace, and the inverse needs what it needed before
+    # every size the one-CTA kernels take needs no forward workspace, and the inverse only its slices
     assert lib.qi_stft_workspace_bytes(3, 100, 8192, _lib.QI_F32) == 0
     assert lib.qi_stft_workspace_bytes(3, 100, 4096, _lib.QI_F64) == 0
     assert lib.qi_stft_workspace_bytes(3, 100, 16384, _lib.QI_F32) == 3 * 50 * (16384 * 8 + 8)
     assert lib.qi_stft_workspace_bytes(3, 101, 8192, _lib.QI_F64) == 3 * 51 * (8192 * 16 + 16)
-    for nfft, code in ((8192, _lib.QI_F32), (4096, _lib.QI_F64), (512, _lib.QI_F64)):
-        assert lib.qi_istft_workspace_bytes_nfft(3, 100, 1000, nfft, code) == lib.qi_istft_workspace_bytes(3, 100, 1000, code)
-    assert lib.qi_istft_workspace_bytes_nfft(3, 100, 9000, 16384, _lib.QI_F32) > lib.qi_istft_workspace_bytes(3, 100, 9000, _lib.QI_F32)
+    for nfft, code, real in ((8192, _lib.QI_F32, 4), (4096, _lib.QI_F64, 8), (512, _lib.QI_F64, 8)):
+        assert lib.qi_istft_workspace_bytes(3, 100, 1000, nfft, code) == 3 * 100 * 1000 * real
+    assert lib.qi_istft_workspace_bytes(3, 100, 9000, 16384, _lib.QI_F32) > 3 * 100 * 9000 * 4
 
     x = record(50000, channels=2, seed=3)
     geom = dict(nperseg=12000, hop=5000, nfft=16384, n_frames=11, pad_left=6000)
@@ -160,12 +161,12 @@ def test_c_abi_workspace_and_chunking(emul):
         assert rc == -2                                                             # QI_ERR_WORKSPACE
         rc, _ = _c_stft(emul, x, dt=dt, ws_bytes=0, ws=False, **geom)
         assert rc == -4                                                             # QI_ERR_UNSUPPORTED
-        # qi_stft itself has no workspace: unchanged
+        # no workspace at all
         win = emul.asarray(np.hanning(16384), dt)
         xs = emul.asarray(x, dt)
         out = emul.empty((2, 8193, 5), "complex128" if dt == "float64" else "complex64")
         assert lib.qi_stft(emul.ptr(xs), 2, 50000, 50000, emul.ptr(win), 16384, 8192, 16384, 5, 8192, 1.0, 1, 0, code,
-                           emul.ptr(out), None, None) == -4
+                           emul.ptr(out), None, None, 0, None) == -4
 
 
 def test_non_pow2_nfft_still_refused(emul):
@@ -174,7 +175,7 @@ def test_non_pow2_nfft_still_refused(emul):
         styx_fft.stft_complex_pow2(record(40000), FS, 12000, nfft_points=12288)
 
 
-def test_long_frame_kernels_under_address_sanitizer(tmp_path):
+def test_long_frame_route_under_address_sanitizer(tmp_path):
     if shutil.which("g++") is None:
         pytest.skip("no g++")
     asan = subprocess.run(["gcc", "-print-file-name=libasan.so"], capture_output=True, text=True).stdout.strip()

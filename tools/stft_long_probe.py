@@ -43,7 +43,7 @@ def forced_long_lib():
                     os.path.join(CSRC, "qi_stft.cu"), os.path.join(CSRC, "qi_capi.cu"), "-o", out],
                    check=True, capture_output=True)
     lib = ctypes.CDLL(out)
-    for name in ("qi_stft_ws", "qi_stft_workspace_bytes"):
+    for name in ("qi_stft", "qi_stft_workspace_bytes"):
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = _lib.SIGNATURES[name]
     return lib
@@ -72,9 +72,9 @@ class Case:
 
     def __call__(self):
         p = lambda t: None if t is None else t.data_ptr()              # noqa: E731
-        rc = self.lib.qi_stft_ws(p(self.x), C, N, N, p(self.win), self.nfft, self.nfft // 2, self.nfft, self.n_frames,
-                                 self.pad_left, 1.0, 1, 0, self.code, p(self.out), p(self.acc), p(self.ws),
-                                 self.ws_bytes, self.rt.stream())
+        rc = self.lib.qi_stft(p(self.x), C, N, N, p(self.win), self.nfft, self.nfft // 2, self.nfft, self.n_frames,
+                              self.pad_left, 1.0, 1, 0, self.code, p(self.out), p(self.acc), p(self.ws),
+                              self.ws_bytes, self.rt.stream())
         assert rc == 0, rc
 
 
